@@ -81,3 +81,25 @@ def test_gpu_arm_prints_one_json_line_with_roofline_and_e2e():
     assert r["bound"] in ("tensor", "fp32", "mufu") and r["unit"] in ("TFLOP/s", "Gop/s")
     assert 0 < r["frac"] < 1 and abs(r["frac"] - r["achieved"] / r["peak"]) < 1e-9 and r["traffic"] > 0
     assert set(d["clocks"]) >= {"sm_mhz", "sm_max_mhz", "reasons"}
+
+
+@pytest.mark.gpu
+def test_gpu_arm_dumps_the_last_timed_step_the_same_way_twice(tmp_path):
+    """--dump-outputs: the rows the last timed step retained and the chain state it left, float32 / float64,
+    64 MB at most (a sample of the 1,024 chains at config 3), and identical from two runs with the same arguments."""
+    import numpy
+    args = ["--steps", "2", "--warmup", "1", "--no-full-run", "--no-sub-records", "--no-cpu-baseline"]
+    dumps = []
+    for k in range(2):
+        out = tmp_path / str(k)
+        _run(args + ["--dump-outputs", str(out)], 600)
+        dumps.append(dict((f[:-4], numpy.load(str(out / f))) for f in os.listdir(str(out))))
+    a, b = dumps
+    assert set(a) == set(b) == {"samples", "theta", "scale", "lprior", "ll", "mu", "sigma2"}
+    assert sum(v.nbytes for v in a.values()) <= 64e6
+    nC = a["theta"].shape[2]
+    assert 0 < nC < 1024 and a["theta"].shape == (9, 1024, nC) and a["ll"].shape == (1024, nC)
+    assert a["samples"].shape == (5, 9 * 1026, nC) and a["mu"].shape == a["sigma2"].shape == (9, nC)   # iterations 100..140
+    for name in a:
+        assert a[name].dtype in (numpy.float32, numpy.float64), name
+        numpy.testing.assert_array_equal(a[name], b[name], err_msg=name)
