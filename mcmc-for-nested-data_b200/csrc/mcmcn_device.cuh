@@ -27,18 +27,6 @@ namespace mcmcn {
 
 #define MCMCN_LOG_SQRT_2PI 0.91893853320467274178  /* numpy.log(numpy.sqrt(2*numpy.pi)) */
 
-// Build switches, each the kept side of a measured A/B (tools/variant.sh builds the other side; results are
-// bit-identical either way except MCMCN_LOGIT_PAIRS, which reorders the FP32 sums of the logit loop):
-#ifndef MCMCN_HYPER_EARLY_DRAWS
-#define MCMCN_HYPER_EARLY_DRAWS 1      /* one-pass Gibbs kernel: the two draws before the sums (18.3 -> 16.9 us at config 3) */
-#endif
-#ifndef MCMCN_PREFETCH_NEXT_GROUP
-#define MCMCN_PREFETCH_NEXT_GROUP 1    /* FP32-pipe step kernel: next group's state and next sweep's log-prior into L1 */
-#endif
-#ifndef MCMCN_LOGIT_PAIRS
-#define MCMCN_LOGIT_PAIRS 1            /* Bernoulli-logit loop as packed FFMA2 over observation pairs */
-#endif
-
 // ---------------------------------------------------------------- small PTX helpers
 __device__ __forceinline__ unsigned smem_u32(const void* p) {
     return (unsigned)__cvta_generic_to_shared(p);
@@ -244,6 +232,93 @@ __device__ __forceinline__ double prior_logpdf(const mcmcn_prior& pr, double x) 
     return __dsub_rn(r, pr.log_scale);
 }
 
+// ---------------------------------------------------------------- sampler rules
+// One copy of each rule of Parameter.step / Parameter.tune, called by every step kernel (sweep_kernel,
+// sweep_tc_kernel, the complete-pooling split) so that they cannot drift apart.
+
+// numpy.random.normal(value, sd), posteriorSampling.py:304-306
+__device__ __forceinline__ double propose(double cur, double sd, double z) {
+    return __dadd_rn(cur, __dmul_rn(sd, z));
+}
+
+// The random numbers of sweeps p and p + 1 (p even) of one chain and group: one Philox4x32-10 call at
+// counter (p >> 1) * G + g, Box-Muller on words 0-1 (cosine branch: sweep p, sine branch: sweep p + 1),
+// words 2 and 3 one accept uniform each (uniform_from32).
+struct SweepDraws {
+    float z0, z1;
+    unsigned u0, u1;
+};
+__device__ __forceinline__ SweepDraws sweep_draws(long long chain_id, unsigned long long seed, long long iter, int p, int G,
+                                                  int g) {
+    const uint4 r = philox_draw(chain_id, seed, iter, MCMCN_STREAM_SWEEP, (unsigned)((p >> 1) * G + g), 1u);
+    SweepDraws d;
+    normal_pair_from(r.x, r.y, d.z0, d.z1);
+    d.u0 = r.z;
+    d.u1 = r.w;
+    return d;
+}
+
+// The decision tree of Parameter.step, :334-367, in two parts.  The fast part returns the decision and sets
+// `exact` when log(u) against diff is too close to call in FP32 (about once per 10^5 decisions); then
+// `decide_exact` settles it with the FP64 logarithm.
+__device__ __forceinline__ bool decide_fast(double post_cur, double post_prop, double llp, double diff, double u, bool& exact) {
+    const bool b1 = !finite64(post_cur) && finite64(post_prop);
+    const bool test = finite64(llp) && finite64(diff);                 // branches 4/5 draw the uniform
+    const int fast = log_u_vs_diff_fast(u, diff);
+    exact = !b1 && test && fast == 0;
+    return b1 || (test && fast > 0);
+}
+__device__ __forceinline__ bool decide_exact(double u, double diff) { return log(u) < diff; }
+
+// Replay machinery of one iteration: the tapes replace the random numbers (z, u) and the decisions, the
+// trace arrays record each decision's inputs.  Null pointers: not in use.
+struct StepTapes {
+    const double* tape_z;
+    const double* tape_u;
+    const unsigned char* tape_acc;
+    double* tr_ll;
+    double* tr_lp;
+    double* tr_diff;
+    unsigned char* tr_acc;
+};
+// Records the decision at element `at` when `record`, and returns the taped decision when `force`.
+__device__ __forceinline__ bool trace_and_force(const StepTapes& t, size_t at, bool record, bool force, double llp,
+                                                double lp_prop, double diff, bool accept) {
+    if (record) {
+        t.tr_ll[at] = llp;
+        t.tr_lp[at] = lp_prop;
+        t.tr_diff[at] = diff;
+        t.tr_acc[at] = accept ? 1 : 0;
+    }
+    if (force) accept = t.tape_acc[at] != 0;
+    return accept;
+}
+
+// Burn-in bookkeeping of one decision: `cnt` packs accepted | rejected << 16 since the last tune; on a tune
+// iteration Parameter.tune (:385-437) scales the step size by the acceptance rate and the count restarts.
+__device__ __forceinline__ unsigned count_and_tune(unsigned cnt, bool accept, bool tune, double* scale) {
+    cnt += accept ? 1u : 0x10000u;
+    if (tune) {
+        const unsigned na = cnt & 0xFFFFu, nr = cnt >> 16;
+        if (na + nr) {
+            const double sc = *scale;
+            const double rate = (double)na / (double)(na + nr);
+            double f = 1.0;
+            if (rate < 0.001) f = 0.1;
+            else if (rate < 0.05) f = 0.5;
+            else if (rate < 0.2) f = 0.9;
+            else if (rate > 0.95) f = 10.0;
+            else if (rate > 0.75) f = 2.0;
+            else if (rate > 0.5) f = 1.1;
+            double ns = __dmul_rn(sc, f);
+            if (ns == 0.0) ns = sc;
+            *scale = ns;
+            cnt = 0;
+        }
+    }
+    return cnt;
+}
+
 // ---------------------------------------------------------------- objective policies
 // A policy restates one reference-style objective as a device function over a group's packed
 // block in shared memory.
@@ -342,6 +417,18 @@ __device__ __forceinline__ float sum2(f32x2 v) {
     asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v));
     return lo + hi;
 }
+
+// The per-chain terms of a policy whose group log-likelihood is the accumulator itself (all but LinReg).
+struct NoAux {
+    struct Aux {};
+    static constexpr int AUX_DOUBLES = 0;
+    __device__ static __forceinline__ void aux_put(const Aux&, double*, int) {}
+    __device__ static __forceinline__ Aux aux_get(const double*, int) { return Aux(); }
+    template <int C, typename T, class W>
+    __device__ static __forceinline__ Aux aux(int, const W&, int) { return Aux(); }
+    __device__ static __forceinline__ bool aux_depends_on(int) { return false; }
+    __device__ static __forceinline__ double finish(double acc, const Aux&) { return acc; }
+};
 
 // Linear regression with K coefficients and a noise sd (example/regression.py:53-67):
 //   ll_i = norm(loc=y_i, scale=sigma).logpdf(x_i . b)
@@ -493,14 +580,12 @@ __device__ __forceinline__ float softplus_t(float eta) {
 __device__ __forceinline__ double softplus_t(double eta) {
     return fmax(eta, 0.0) + log1p(exp(-fabs(eta)));
 }
-#ifndef MCMCN_LOGIT_FOLD_QUADS
-#define MCMCN_LOGIT_FOLD_QUADS 16
-#endif
-struct Logit {
+struct Logit : NoAux {
     static constexpr int P = 2;
     static constexpr int UNIT = 8;
     static constexpr int HDR = 0;
     static constexpr int OBS_PER_UNIT = 4;
+    static constexpr int FOLD_QUADS = 16;        // quads per FP64 fold of the FP32 loop
 
     template <typename T>
     __device__ static __forceinline__ T local(int, double v, const double*, int) { return (T)v; }
@@ -532,7 +617,6 @@ struct Logit {
     // each), and four FFMA (e; product *= 1 + t; two for the linear part) instead of seven FP32 ops.
     // The product of 16 factors carries 16 roundings of 6e-8 relative, i.e. the same absolute error
     // in the logarithm as the sum of 16 rounded logarithms had.
-#if MCMCN_LOGIT_PAIRS
     // Production form of the loop above: the same four FMAs and one ex2 per evaluation, issued for TWO
     // observations of one chain at a time as packed FFMA2 (e; product *= 1 + t; s += (y - 1/2) e), the pair
     // (x_j, x_j+1) being an aligned register pair of the 128-bit shared load as it is; only the |e| / 2 term
@@ -596,12 +680,12 @@ struct Logit {
         const float* xr = blk + (size_t)nq * UNIT;
         if (rem & 2) MCMCN_LOGIT_PAIR(pack2(xr[0], xr[1]), pack2(xr[4], xr[5]))
         if (rem & 1) MCMCN_LOGIT_ONE(xr[rem - 1], xr[4 + rem - 1])
-        // MCMCN_LOGIT_FOLD_QUADS quads per fold: one lg2 and one FP32 -> FP64 conversion (both XU operations) per
+        // FOLD_QUADS quads per fold: one lg2 and one FP32 -> FP64 conversion (both XU operations) per
         // fold and chain.  16 quads: each half's product of up to 34 factors in (1, 2] and the product of the two
         // halves stay below 2^67; their roundings (4e-6 relative) move the logarithm by 6e-6 absolute -- against
         // group log-likelihoods of tens, inside the 1e-5 relative bar with a wide margin.
-        for (int q0 = 0; q0 < nq; q0 += MCMCN_LOGIT_FOLD_QUADS) {
-            const int qend = min(nq, q0 + MCMCN_LOGIT_FOLD_QUADS);
+        for (int q0 = 0; q0 < nq; q0 += FOLD_QUADS) {
+            const int qend = min(nq, q0 + FOLD_QUADS);
             for (int q1 = q0; q1 < qend; q1 += 4) {
 #pragma unroll
                 for (int u = 0; u < 4; ++u) {
@@ -621,66 +705,6 @@ struct Logit {
 #undef MCMCN_LOGIT_ONE
 #undef MCMCN_LOGIT_FOLD
     }
-#else
-    template <int C>
-    __device__ static __forceinline__ void all_obs(const float* __restrict__ blk, int nobs, const Work<C, float>& w, double (&acc)[C]) {
-        const int nq = nobs >> 2, rem = nobs & 3;
-        float a2[C], b2[C], s[C], pr[C];
-#pragma unroll
-        for (int c = 0; c < C; ++c) {
-            a2[c] = w.th[c][0] * 1.4426950408889634f;
-            b2[c] = w.th[c][1] * 1.4426950408889634f;
-            s[c] = 0.0f;
-            pr[c] = 1.0f;
-        }
-#define MCMCN_LOGIT_OBS(xv, yv)                                                          \
-        {                                                                                \
-            const float yh = (yv) - 0.5f;                                                \
-            _Pragma("unroll") for (int c = 0; c < C; ++c) {                              \
-                const float e = fmaf(b2[c], (xv), a2[c]);                                \
-                float t;                                                                 \
-                asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(t) : "f"(-fabsf(e)));            \
-                pr[c] = fmaf(pr[c], t, pr[c]);                                           \
-                s[c] = fmaf(yh, e, s[c]);                                                \
-                s[c] = fmaf(-0.5f, fabsf(e), s[c]);                                      \
-            }                                                                            \
-        }
-#define MCMCN_LOGIT_FOLD()                                                               \
-        _Pragma("unroll") for (int c = 0; c < C; ++c) {                                  \
-            float l;                                                                     \
-            asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(l) : "f"(pr[c]));                    \
-            acc[c] += (double)(0.6931471805599453f * (s[c] - l));                        \
-            s[c] = 0.0f;                                                                 \
-            pr[c] = 1.0f;                                                                \
-        }
-        // the 1-3 observations of the last, partial quad join the first fold (at most 19 factors)
-        const float* xr = blk + (size_t)nq * UNIT;
-        for (int j = 0; j < rem; ++j) MCMCN_LOGIT_OBS(xr[j], xr[4 + j])
-        // MCMCN_LOGIT_FOLD_QUADS quads (x 4 observations) per fold: one lg2 and one FP32 -> FP64 conversion (both on
-        // the XU pipe that bounds this loop) per fold and chain.  16 quads: the product of up to 67 factors in
-        // (1, 2] stays below 2^67, and its 67 roundings (4e-6 relative) move the logarithm by 6e-6 absolute --
-        // against group log-likelihoods of tens, inside the 1e-5 relative bar with a wide margin.
-        for (int q0 = 0; q0 < nq; q0 += MCMCN_LOGIT_FOLD_QUADS) {
-            const int qend = min(nq, q0 + MCMCN_LOGIT_FOLD_QUADS);
-            for (int q1 = q0; q1 < qend; q1 += 4) {
-#pragma unroll
-                for (int u = 0; u < 4; ++u) {
-                    if (q1 + u < qend) {
-                        float x4[4], y4[4];
-                        Vec4<float>::load(blk + (size_t)(q1 + u) * UNIT, x4);
-                        Vec4<float>::load(blk + (size_t)(q1 + u) * UNIT + 4, y4);
-#pragma unroll
-                        for (int j = 0; j < 4; ++j) MCMCN_LOGIT_OBS(x4[j], y4[j])
-                    }
-                }
-            }
-            MCMCN_LOGIT_FOLD()
-        }
-        if (nq == 0) MCMCN_LOGIT_FOLD()
-#undef MCMCN_LOGIT_OBS
-#undef MCMCN_LOGIT_FOLD
-    }
-#endif
     template <int C>
     __device__ static __forceinline__ void all_obs(const double* __restrict__ blk, int nobs, const Work<C, double>& w, double (&acc)[C]) {
         const int nq = nobs >> 2, rem = nobs & 3;
@@ -700,14 +724,6 @@ struct Logit {
                                                       const Work<C, T>& w, double (&acc)[C], const ObsCtx&) {
         all_obs<C>(blk, nobs, w, acc);
     }
-    struct Aux {};
-    static constexpr int AUX_DOUBLES = 0;
-    __device__ static __forceinline__ void aux_put(const Aux&, double*, int) {}
-    __device__ static __forceinline__ Aux aux_get(const double*, int) { return Aux(); }
-    template <int C, typename T>
-    __device__ static __forceinline__ Aux aux(int, const Work<C, T>&, int) { return Aux(); }
-    __device__ static __forceinline__ bool aux_depends_on(int) { return false; }
-    __device__ static __forceinline__ double finish(double acc, const Aux&) { return acc; }
     template <typename T>
     __device__ static __forceinline__ double pointwise(const T* __restrict__ blk, int i, const double*, const T (&th)[P], int = 0, const void* = nullptr) {
         const T* xq = blk + (size_t)(i >> 2) * UNIT;
@@ -723,7 +739,7 @@ struct Logit {
 // packed record of observation i carries its own mu_j[g(i)].
 // Block: ceil(R/4) quads of [4 obs][PP] mu, PP = P rounded up to 4.  obj_const = sd[P] then log(sd)[P].
 template <int P_>
-struct GaussDist {
+struct GaussDist : NoAux {
     static constexpr int P = P_;
     static constexpr int PP = (P_ + 3) & ~3;
     static constexpr int UNIT = 4 * PP;
@@ -754,14 +770,6 @@ struct GaussDist {
             for (int c = 0; c < C; ++c) acc[c] = __dadd_rn(acc[c], (double)row<T>(rec, cst, w.th[c]));
         }
     }
-    struct Aux {};
-    static constexpr int AUX_DOUBLES = 0;
-    __device__ static __forceinline__ void aux_put(const Aux&, double*, int) {}
-    __device__ static __forceinline__ Aux aux_get(const double*, int) { return Aux(); }
-    template <int C, typename T>
-    __device__ static __forceinline__ Aux aux(int, const Work<C, T>&, int) { return Aux(); }
-    __device__ static __forceinline__ bool aux_depends_on(int) { return false; }
-    __device__ static __forceinline__ double finish(double acc, const Aux&) { return acc; }
     template <typename T>
     __device__ static __forceinline__ double pointwise(const T* __restrict__ blk, int i, const double* cst, const T (&th)[P], int = 0, const void* = nullptr) {
         return (double)row<T>(blk + (size_t)(i >> 2) * UNIT + (i & 3) * PP, cst, th);
@@ -774,7 +782,7 @@ struct GaussDist {
 //                                        const mcmc_real* hdr, int obs_index, int group);
 // before including this header.  Block: [HDR] header, then R records of OBS values.
 #ifdef MCMCN_USER_P
-struct UserObj {
+struct UserObj : NoAux {
     static constexpr int P = MCMCN_USER_P;
     static constexpr int UNIT = MCMCN_USER_OBS;
     static constexpr int HDR = MCMCN_USER_HDR;
@@ -795,14 +803,6 @@ struct UserObj {
                 acc[c] += (double)mcmc_obj_loglik(w.th[c], blk + (size_t)i * UNIT, hdr, ctx.obs0 + i, ctx.group);
         }
     }
-    struct Aux {};
-    static constexpr int AUX_DOUBLES = 0;
-    __device__ static __forceinline__ void aux_put(const Aux&, double*, int) {}
-    __device__ static __forceinline__ Aux aux_get(const double*, int) { return Aux(); }
-    template <int C, typename T>
-    __device__ static __forceinline__ Aux aux(int, const Work<C, T>&, int) { return Aux(); }
-    __device__ static __forceinline__ bool aux_depends_on(int) { return false; }
-    __device__ static __forceinline__ double finish(double acc, const Aux&) { return acc; }
     template <typename T>
     __device__ static __forceinline__ double pointwise(const T* __restrict__ blk, int i, const double*, const T (&th)[P],
                                                        int g, const void* hdr) {
@@ -839,13 +839,7 @@ struct SweepArgs {
     long long iter;
     unsigned long long seed;
     int tune, count, use_override;
-    const double* tape_z;
-    const double* tape_u;
-    const unsigned char* tape_acc;
-    double* tr_ll;
-    double* tr_lp;
-    double* tr_diff;
-    unsigned char* tr_acc;
+    StepTapes tp;
     // eval-only mode
     const double* pooled_theta;   // [P][S] or NULL
     double* out_ll;               // [G][S]
@@ -929,9 +923,9 @@ __global__ void __launch_bounds__(MAXT, MINB) sweep_kernel(const SweepArgs a) {
     constexpr bool GENERAL = F < 0;
     const bool partial = GENERAL ? (a.partial != 0) : ((F & MCMCN_F_PARTIAL) != 0);
     const bool count = GENERAL ? (a.count != 0) : ((F & MCMCN_F_COUNT) != 0);
-    const bool replay = GENERAL && a.tape_z != nullptr;
-    const bool trace = GENERAL && a.tr_ll != nullptr;
-    const bool forced = GENERAL && a.tape_acc != nullptr;
+    const bool replay = GENERAL && a.tp.tape_z != nullptr;
+    const bool trace = GENERAL && a.tp.tr_ll != nullptr;
+    const bool forced = GENERAL && a.tp.tape_acc != nullptr;
     const bool override_lp = GENERAL && a.use_override != 0;
 
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -1006,12 +1000,9 @@ __global__ void __launch_bounds__(MAXT, MINB) sweep_kernel(const SweepArgs a) {
                             prefetch_l1(a.hyper + ((size_t)3 * P + p + 1) * S + chl[c]);
                             prefetch_l1(a.hyper + ((size_t)4 * P + p + 1) * S + chl[c]);
                         }
-#if MCMCN_PREFETCH_NEXT_GROUP
                         else prefetch_l1(a.lprior + row + (size_t)a.G * S + chl[c]);
-#endif
                     }
                 }
-#if MCMCN_PREFETCH_NEXT_GROUP
                 else if (g + 1 < g1) {                                 // last sweep of the group: the next group's state, which
 #pragma unroll                                                         // the group prologue and its first sweep read, into L1
                     for (int c = 0; c < C; ++c) {
@@ -1024,29 +1015,20 @@ __global__ void __launch_bounds__(MAXT, MINB) sweep_kernel(const SweepArgs a) {
                         if (!partial) prefetch_l1(a.lprior + nx);
                     }
                 }
-#endif
                 if (replay) {
 #pragma unroll
                     for (int c = 0; c < C; ++c) {
-                        z[c] = a.tape_z[row + chl[c]];
-                        uu[c] = a.tape_u[row + chl[c]];
+                        z[c] = a.tp.tape_z[row + chl[c]];
+                        uu[c] = a.tp.tape_u[row + chl[c]];
                     }
                 } else if ((p & 1) == 0) {
-                    // One Philox4x32-10 call per two sweeps, the recipe of the tcgen05 step kernel (same
-                    // counters, same draws): words 0-1 -> two normals, words 2, 3 -> one uniform each;
-                    // the odd sweep's pair waits in a parking slot as (float z, 32-bit word).
-                    uint4 rnd[C];
-#pragma unroll
-                    for (int c = 0; c < C; ++c)
-                        rnd[c] = philox_draw(a.chain_id0 + chl[c], a.seed, a.iter, MCMCN_STREAM_SWEEP,
-                                             (unsigned)((p >> 1) * a.G + g), 1u);
+                    // the odd sweep's draws wait in a parking slot as (float z, 32-bit word)
 #pragma unroll
                     for (int c = 0; c < C; ++c) {
-                        float zc, zs;
-                        normal_pair_from(rnd[c].x, rnd[c].y, zc, zs);
-                        z[c] = (double)zc;
-                        uu[c] = uniform_from32(rnd[c].z);
-                        SLOT(ST_RAND2, c) = __hiloint2double((int)rnd[c].w, __float_as_int(zs));
+                        const SweepDraws d = sweep_draws(a.chain_id0 + chl[c], a.seed, a.iter, p, a.G, g);
+                        z[c] = (double)d.z0;
+                        uu[c] = uniform_from32(d.u0);
+                        SLOT(ST_RAND2, c) = __hiloint2double((int)d.u1, __float_as_int(d.z1));
                     }
                 } else {
 #pragma unroll
@@ -1057,8 +1039,7 @@ __global__ void __launch_bounds__(MAXT, MINB) sweep_kernel(const SweepArgs a) {
                     }
                 }
 #pragma unroll
-                for (int c = 0; c < C; ++c)
-                    prop[c] = __dadd_rn(cur[c], __dmul_rn(sc[c], z[c]));   // numpy.random.normal(value, sd), :304-306
+                for (int c = 0; c < C; ++c) prop[c] = propose(cur[c], sc[c], z[c]);
                 // log-priors of the proposal and of the current value (pure functions of state
                 // known now; the reference evaluates them after the likelihood, :335, :331)
                 double lp_prop[C], lp_cur[C];
@@ -1103,7 +1084,10 @@ __global__ void __launch_bounds__(MAXT, MINB) sweep_kernel(const SweepArgs a) {
 #pragma unroll
                 for (int c = 0; c < C; ++c) aux_prop[c] = Obj::template aux<C, T>(R, w, c);
             }
-            // Parameter.step decision tree, :334-367
+            // decide_fast / decide_exact over C chains, written out here: the exact test is hoisted out of the
+            // chain loop (one rare branch for all C chains), and its short-circuit recomputation of decide_fast's
+            // `exact` keeps the observation loop's register allocation (through the function it moves by 1-4
+            // registers and adds spills in some linear-regression instantiations)
             double llp[C], diff[C], uu[C], lp_prop[C], post_cur[C];
             bool acc_own[C];
             bool exact_any = false;
@@ -1129,23 +1113,15 @@ __global__ void __launch_bounds__(MAXT, MINB) sweep_kernel(const SweepArgs a) {
                 for (int c = 0; c < C; ++c) {
                     const bool b1 = !finite64(post_cur[c]) && finite64(lp_prop[c] + llp[c]);
                     if (!b1 && finite64(llp[c]) && finite64(diff[c]) && log_u_vs_diff_fast(uu[c], diff[c]) == 0)
-                        acc_own[c] = log(uu[c]) < diff[c];
+                        acc_own[c] = decide_exact(uu[c], diff[c]);
                 }
             }
 #pragma unroll
             for (int c = 0; c < C; ++c) {
                 const size_t at = row + chl[c];
                 bool accept = acc_own[c];
-                if (GENERAL) {
-                    if (trace && on[c]) {
-                        a.tr_ll[at] = llp[c];
-                        a.tr_lp[at] = lp_prop[c];
-                        a.tr_diff[at] = diff[c];
-                        a.tr_acc[at] = acc_own[c] ? 1 : 0;
-                    }
-                    if (forced) accept = a.tape_acc[at] != 0;
-                }
-                if (accept) {                                        // :369-378, :608-610
+                if (GENERAL) accept = trace_and_force(a.tp, at, trace && on[c], forced, llp[c], lp_prop[c], diff[c], accept);
+                if (accept) {                                      // :369-378, :608-610
                     if (on[c]) {
                         a.theta[at] = SLOT(ST_PROP, c);
                         if (!partial) a.lprior[at] = lp_prop[c];
@@ -1155,29 +1131,7 @@ __global__ void __launch_bounds__(MAXT, MINB) sweep_kernel(const SweepArgs a) {
                 } else {
                     w.set(c, p, (T)SLOT(ST_OLD, c));
                 }
-                if (count && on[c]) {
-                    unsigned cnt = a.counts[at];
-                    cnt += accept ? 1u : 0x10000u;
-                    if (a.tune) {                                    // Parameter.tune, :385-437
-                        const unsigned na = cnt & 0xFFFFu, nr = cnt >> 16;
-                        if (na + nr) {
-                            const double sc = a.scale[at];
-                            const double rate = (double)na / (double)(na + nr);
-                            double f = 1.0;
-                            if (rate < 0.001) f = 0.1;
-                            else if (rate < 0.05) f = 0.5;
-                            else if (rate < 0.2) f = 0.9;
-                            else if (rate > 0.95) f = 10.0;
-                            else if (rate > 0.75) f = 2.0;
-                            else if (rate > 0.5) f = 1.1;
-                            double ns = __dmul_rn(sc, f);
-                            if (ns == 0.0) ns = sc;
-                            a.scale[at] = ns;
-                            cnt = 0;
-                        }
-                    }
-                    a.counts[at] = cnt;
-                }
+                if (count && on[c]) a.counts[at] = count_and_tune(a.counts[at], accept, a.tune, a.scale + at);
             }
         }
 #pragma unroll
@@ -1300,6 +1254,39 @@ __device__ inline double gamma_draw(double a, long long chain_id, unsigned long 
     return g;
 }
 
+// The two draws of HyperParameter.update for (name p, chain ch), from the tapes when replaying: the standard
+// normal of the mu draw (:487) and the unit inverse-gamma of the sigma2 draw (:497-498).
+__device__ __forceinline__ double hyper_z(const HyperArgs& a, int p, int ch) {
+    if (a.tape_zmu) return a.tape_zmu[(size_t)p * a.S + ch];
+    const uint4 r = philox_draw(a.chain_id0 + ch, a.seed, a.iter, MCMCN_STREAM_HYPER, (unsigned)p, 0u);
+    return normal_from(r.x, r.y);
+}
+__device__ __forceinline__ double hyper_q(const HyperArgs& a, int p, int ch) {
+    if (a.tape_qsig) return a.tape_qsig[(size_t)p * a.S + ch];
+    return 1.0 / gamma_draw(((double)a.G - 1.0) / 2.0, a.chain_id0 + ch, a.seed, a.iter, (unsigned)p);
+}
+// mu = muHat + sqrt(sigma2_old / G) z, :485-487
+__device__ __forceinline__ double hyper_mu(const HyperArgs& a, int p, int ch, double muHat, double z) {
+    const double sigma2_old = a.hyper[((size_t)1 * a.P + p) * a.S + ch];
+    const double sd = sqrt(sigma2_old / (double)a.G);                       // :486
+    return __dadd_rn(muHat, __dmul_rn(sd, z));
+}
+// sigma2 from the sum of squares about the new mu and the unit inverse-gamma draw q (:494-498), then the five
+// rows of hyper: mu, sigma2, sd, log sd, 1 / sd (getDistribution :500-502)
+__device__ __forceinline__ void hyper_finish(const HyperArgs& a, int p, int ch, double mu, double ss, double q) {
+    const double n = (double)a.G;
+    const double hat = ss / (n - 1.0);
+    const double aa = (n - 1.0) / 2.0;
+    const double sigma2 = __dadd_rn(__dmul_rn(q, __dmul_rn(aa, hat)), 0.0);
+    const double sd = sqrt(sigma2);
+    const size_t S = (size_t)a.S;
+    a.hyper[((size_t)0 * a.P + p) * S + ch] = mu;
+    a.hyper[((size_t)1 * a.P + p) * S + ch] = sigma2;
+    a.hyper[((size_t)2 * a.P + p) * S + ch] = sd;
+    a.hyper[((size_t)3 * a.P + p) * S + ch] = log(sd);
+    a.hyper[((size_t)4 * a.P + p) * S + ch] = 1.0 / sd;
+}
+
 template <int NS>
 __global__ void __launch_bounds__(32 * NS) hyper_kernel(const HyperArgs a) {
     __shared__ double red[NS][33];
@@ -1321,20 +1308,7 @@ __global__ void __launch_bounds__(32 * NS) hyper_kernel(const HyperArgs a) {
         double t = 0.0;
 #pragma unroll
         for (int k = 0; k < NS; ++k) t += red[k][tx];
-        double mu = 0.0;
-        if (on) {
-            const double muHat = t / n;
-            const double sigma2_old = a.hyper[((size_t)1 * a.P + p) * S + ch];
-            const double sd = sqrt(sigma2_old / n);                               // :486
-            double z;
-            if (a.tape_zmu) z = a.tape_zmu[(size_t)p * S + ch];
-            else {
-                const uint4 r = philox_draw(a.chain_id0 + ch, a.seed, a.iter, MCMCN_STREAM_HYPER, (unsigned)p, 0u);
-                z = normal_from(r.x, r.y);
-            }
-            mu = __dadd_rn(muHat, __dmul_rn(sd, z));                               // :487
-        }
-        mu_s[tx] = mu;
+        mu_s[tx] = on ? hyper_mu(a, p, ch, t / n, hyper_z(a, p, ch)) : 0.0;
     }
     __syncthreads();
     // pass 2: sum of squares about the NEW mu (:494)
@@ -1348,18 +1322,7 @@ __global__ void __launch_bounds__(32 * NS) hyper_kernel(const HyperArgs a) {
         double ss = 0.0;
 #pragma unroll
         for (int k = 0; k < NS; ++k) ss += red[k][tx];
-        const double hat = ss / (n - 1.0);
-        const double aa = (n - 1.0) / 2.0;
-        double q;                                                                   // unit inverse-gamma draw, :497-498
-        if (a.tape_qsig) q = a.tape_qsig[(size_t)p * S + ch];
-        else q = 1.0 / gamma_draw(aa, a.chain_id0 + ch, a.seed, a.iter, (unsigned)p);
-        const double sigma2 = __dadd_rn(__dmul_rn(q, __dmul_rn(aa, hat)), 0.0);
-        const double sd = sqrt(sigma2);
-        a.hyper[((size_t)0 * a.P + p) * S + ch] = mu;
-        a.hyper[((size_t)1 * a.P + p) * S + ch] = sigma2;
-        a.hyper[((size_t)2 * a.P + p) * S + ch] = sd;
-        a.hyper[((size_t)3 * a.P + p) * S + ch] = log(sd);
-        a.hyper[((size_t)4 * a.P + p) * S + ch] = 1.0 / sd;
+        hyper_finish(a, p, ch, mu, ss, hyper_q(a, p, ch));
     }
 }
 
@@ -1390,19 +1353,14 @@ __global__ void __launch_bounds__(CX * (MCMCN_HYPER_SLICES / SPR)) hyper_onepass
         c = a.hyper[((size_t)0 * a.P + p) * S + ch];
         if (!finite64(c)) c = th[0];
     }
-#if MCMCN_HYPER_EARLY_DRAWS
     // The two random draws of this (name, chain) do not depend on the sums: the finishing row forms them before
     // its loads, under the other rows' memory latency, instead of after the block's barrier (a serial tail of
     // Philox, Box-Muller, Marsaglia-Tsang and FP64 logarithms with the rest of the GPU idle).
-    double z_early = 0.0, q_early = 0.0;
+    double z = 0.0, q = 0.0;
     if (ty == 0 && on) {
-        if (!a.tape_zmu) {
-            const uint4 r = philox_draw(a.chain_id0 + ch, a.seed, a.iter, MCMCN_STREAM_HYPER, (unsigned)p, 0u);
-            z_early = normal_from(r.x, r.y);
-        }
-        if (!a.tape_qsig) q_early = 1.0 / gamma_draw((n - 1.0) / 2.0, a.chain_id0 + ch, a.seed, a.iter, (unsigned)p);
+        z = hyper_z(a, p, ch);
+        q = hyper_q(a, p, ch);
     }
-#endif
 #pragma unroll
     for (int q = 0; q < SPR; ++q) {
         const int slice = ty * SPR + q;
@@ -1440,37 +1398,9 @@ __global__ void __launch_bounds__(CX * (MCMCN_HYPER_SLICES / SPR)) hyper_onepass
         for (int k = 0; k < NS; ++k) { t1 += red1[k][tx]; t2 += red2[k][tx]; }
         const double dmean = t1 / n;
         const double muHat = c + dmean;                                           // numpy.mean, :485
-        const double sigma2_old = a.hyper[((size_t)1 * a.P + p) * S + ch];
-        const double sdm = sqrt(sigma2_old / n);                                  // :486
-        double z;
-        if (a.tape_zmu) z = a.tape_zmu[(size_t)p * S + ch];
-        else {
-#if MCMCN_HYPER_EARLY_DRAWS
-            z = z_early;
-#else
-            const uint4 r = philox_draw(a.chain_id0 + ch, a.seed, a.iter, MCMCN_STREAM_HYPER, (unsigned)p, 0u);
-            z = normal_from(r.x, r.y);
-#endif
-        }
-        const double mu = __dadd_rn(muHat, __dmul_rn(sdm, z));                    // :487
+        const double mu = hyper_mu(a, p, ch, muHat, z);
         const double dmu = mu - muHat;
-        const double ss = fma(n * dmu, dmu, fmax(fma(-dmean, t1, t2), 0.0));      // :494
-        const double hat = ss / (n - 1.0);
-        const double aa = (n - 1.0) / 2.0;
-        double q;                                                                 // unit inverse-gamma draw, :497-498
-        if (a.tape_qsig) q = a.tape_qsig[(size_t)p * S + ch];
-#if MCMCN_HYPER_EARLY_DRAWS
-        else q = q_early;
-#else
-        else q = 1.0 / gamma_draw(aa, a.chain_id0 + ch, a.seed, a.iter, (unsigned)p);
-#endif
-        const double sigma2 = __dadd_rn(__dmul_rn(q, __dmul_rn(aa, hat)), 0.0);
-        const double sd = sqrt(sigma2);
-        a.hyper[((size_t)0 * a.P + p) * S + ch] = mu;
-        a.hyper[((size_t)1 * a.P + p) * S + ch] = sigma2;
-        a.hyper[((size_t)2 * a.P + p) * S + ch] = sd;
-        a.hyper[((size_t)3 * a.P + p) * S + ch] = log(sd);
-        a.hyper[((size_t)4 * a.P + p) * S + ch] = 1.0 / sd;
+        hyper_finish(a, p, ch, mu, fma(n * dmu, dmu, fmax(fma(-dmean, t1, t2), 0.0)), q);   // :494
     }
 }
 
@@ -1497,13 +1427,7 @@ struct CompleteArgs {
     double* cand;                 // [P][S] candidate vector: current values, name p replaced by the proposal
     double* part;                 // [n_parts][S] log-likelihood of the candidate per small group
     double* park;                 // [3][S] proposal, uniform, proposal log-prior
-    const double* tape_z;         // [P][1][S] of this iteration, or null
-    const double* tape_u;
-    const unsigned char* tape_acc;
-    double* tr_ll;
-    double* tr_lp;
-    double* tr_diff;
-    unsigned char* tr_acc;
+    StepTapes tp;                 // [P][1][S] arrays of this iteration
 };
 
 // Proposal of name p for chain c (lanes past the last chain redo its work): candidate vector, parked proposal,
@@ -1512,17 +1436,15 @@ __device__ __forceinline__ void complete_propose(const CompleteArgs& a, int p, c
     const int chl = min(c, a.n_chains - 1);
     const size_t S = (size_t)a.S, at = (size_t)p * S + chl;
     double z, u;
-    if (a.tape_z) {
-        z = a.tape_z[at];
-        u = a.tape_u[at];
-    } else {                      // the step kernels' recipe with G = 1: one Philox call per two sweeps
-        const uint4 rnd = philox_draw(a.chain_id0 + chl, a.seed, a.iter, MCMCN_STREAM_SWEEP, (unsigned)(p >> 1), 1u);
-        float zc, zs;
-        normal_pair_from(rnd.x, rnd.y, zc, zs);
-        z = (double)((p & 1) ? zs : zc);
-        u = uniform_from32((p & 1) ? rnd.w : rnd.z);
+    if (a.tp.tape_z) {
+        z = a.tp.tape_z[at];
+        u = a.tp.tape_u[at];
+    } else {                      // the step kernels' draws with G = 1
+        const SweepDraws d = sweep_draws(a.chain_id0 + chl, a.seed, a.iter, p, 1, 0);
+        z = (double)((p & 1) ? d.z1 : d.z0);
+        u = uniform_from32((p & 1) ? d.u1 : d.u0);
     }
-    const double prop = __dadd_rn(a.theta[at], __dmul_rn(a.scale[at], z));   // :304-306
+    const double prop = propose(a.theta[at], a.scale[at], z);
     for (int k = 0; k < a.P; ++k) a.cand[(size_t)k * S + c] = (k == p) ? prop : a.theta[(size_t)k * S + chl];
     a.park[c] = prop;
     a.park[S + c] = u;
@@ -1560,50 +1482,19 @@ static __global__ void __launch_bounds__(1024) complete_decide_kernel(const Comp
 #pragma unroll
     for (int j = 0; j < 32; ++j) llp += slice_sum[j][threadIdx.x];
     const double prop = a.park[c], u = a.park[S + c], lp_prop = a.park[2 * S + c];
-    // Parameter.step decision tree, :334-367
     const double post_prop = lp_prop + llp;
     const double post_cur = a.lprior[at] + a.ll[c];
     const double diff = post_prop - post_cur;
-    const bool b1 = !finite64(post_cur) && finite64(post_prop);
-    const bool test = finite64(llp) && finite64(diff);                 // branches 4/5 draw the uniform
-    const int fast = log_u_vs_diff_fast(u, diff);
-    bool accept = b1 || (test && fast > 0);
-    if (!b1 && test && fast == 0) accept = log(u) < diff;
-    if (a.tr_ll) {
-        a.tr_ll[at] = llp;
-        a.tr_lp[at] = lp_prop;
-        a.tr_diff[at] = diff;
-        a.tr_acc[at] = accept ? 1 : 0;
-    }
-    if (a.tape_acc) accept = a.tape_acc[at] != 0;
+    bool exact;
+    bool accept = decide_fast(post_cur, post_prop, llp, diff, u, exact);
+    if (exact) accept = decide_exact(u, diff);
+    accept = trace_and_force(a.tp, at, a.tp.tr_ll != nullptr, a.tp.tape_acc != nullptr, llp, lp_prop, diff, accept);
     if (accept) {                                                       // :369-378
         a.theta[at] = prop;
         a.lprior[at] = lp_prop;
         a.ll[c] = llp;
     }
-    if (a.count) {
-        unsigned cnt = a.counts[at];
-        cnt += accept ? 1u : 0x10000u;
-        if (a.tune) {                                                   // Parameter.tune, :385-437
-            const unsigned na = cnt & 0xFFFFu, nr = cnt >> 16;
-            if (na + nr) {
-                const double sc = a.scale[at];
-                const double rate = (double)na / (double)(na + nr);
-                double f = 1.0;
-                if (rate < 0.001) f = 0.1;
-                else if (rate < 0.05) f = 0.5;
-                else if (rate < 0.2) f = 0.9;
-                else if (rate > 0.95) f = 10.0;
-                else if (rate > 0.75) f = 2.0;
-                else if (rate > 0.5) f = 1.1;
-                double ns = __dmul_rn(sc, f);
-                if (ns == 0.0) ns = sc;
-                a.scale[at] = ns;
-                cnt = 0;
-            }
-        }
-        a.counts[at] = cnt;
-    }
+    if (a.count) a.counts[at] = count_and_tune(a.counts[at], accept, a.tune, a.scale + at);
     // the next sweep's proposal in the same launch (this chain's own state only; tapes are indexed by name)
     if (a.propose_next) complete_propose(a, a.p + 1, a.prior_next, c);
 }

@@ -208,9 +208,83 @@ static int launch_pointwise(const KernelSet* ks, const mcmcn_model* m, const mcm
     return MCMCN_OK;
 }
 
+// ---------------------------------------------------------------- per-iteration schedule of a run
+// Burn-in bookkeeping of iteration i: tune on every tune_interval-th iteration below burn (but not 0); count
+// accept / reject only up to the last such tune, since tune() is the counters' only reader.
+struct IterFlags { int tune, count; };
+static IterFlags iter_flags(const mcmcn_run_args* r, long long i) {
+    long long last_tune = 0;
+    if (r->burn > 0) last_tune = ((long long)(r->burn - 1) / r->tune_interval) * r->tune_interval;
+    IterFlags f;
+    f.tune = (i != 0 && i < r->burn && (i % r->tune_interval) == 0) ? 1 : 0;
+    f.count = (i <= last_tune) ? 1 : 0;
+    return f;
+}
+
+// The tape and trace arrays of iteration `it` of the call ([P][G][S] each, per_iter = P G S elements).
+static StepTapes iter_tapes(const mcmcn_run_args* r, int it, size_t per_iter) {
+    StepTapes t;
+    t.tape_z = r->tape_z ? r->tape_z + it * per_iter : nullptr;
+    t.tape_u = r->tape_u ? r->tape_u + it * per_iter : nullptr;
+    t.tape_acc = r->tape_accept ? r->tape_accept + it * per_iter : nullptr;
+    t.tr_ll = r->trace_ll ? r->trace_ll + it * per_iter : nullptr;
+    t.tr_lp = r->trace_lp ? r->trace_lp + it * per_iter : nullptr;
+    t.tr_diff = r->trace_diff ? r->trace_diff + it * per_iter : nullptr;
+    t.tr_acc = r->trace_accept ? r->trace_accept + it * per_iter : nullptr;
+    return t;
+}
+
+// Optional per-kernel timing (mcmcn_run_args.timing): every launch of kind k (0 step, 1 Gibbs, 2 snapshot) is
+// counted in timing[3 + k]; on sampled iterations it is also bracketed by an event pair that
+// mcmcn_timing_collect() reads later, so the call stays asynchronous.
+struct KernelTimer {
+    double* timing;
+    cudaStream_t stream;
+    bool sampled;
+    void tic(int kind) {
+        if (!timing) return;
+        timing[3 + kind] += 1.0;
+        if (!sampled) return;
+        Stamp st; st.kind = kind; st.out = timing;
+        cudaEventCreate(&st.e0); cudaEventCreate(&st.e1);
+        cudaEventRecord(st.e0, stream);
+        g_stamps.push_back(st);
+    }
+    void toc() { if (timing && sampled) cudaEventRecord(g_stamps.back().e1, stream); }
+};
+
+// The retained-row write of iteration i, when Sampler._loop keeps it (i >= burn and i % thin == 0, :887,
+// Sampler._printLogLikelihood :890-891, :907-909): the chain state of model m (per name [mu, sigma2 (partial)],
+// theta[0..G-1]) into store row `row`, and with loglik_store the pointwise log-likelihood of the same row.
+static int write_retained_row(const KernelSet* ks, const mcmcn_model* m, const mcmcn_state* s, const mcmcn_run_args* r,
+                              long long i, int64_t& row, KernelTimer& tm, cudaStream_t stream) {
+    if (!r->store || i < r->burn || (i % r->thin) != 0) return MCMCN_OK;
+    if (row >= r->store_rows) { set_error("sample store overflow at row %lld", (long long)row); return MCMCN_ERR_INVALID; }
+    const bool partial = m->pooling == MCMCN_POOL_PARTIAL;
+    const int ncol = m->n_params * (m->n_groups + (partial ? 2 : 0));
+    const size_t S = (size_t)s->stride;
+    const dim3 sg((unsigned)((ncol + MCMCN_SNAP_COLS - 1) / MCMCN_SNAP_COLS), (unsigned)((s->n_chains + 127) / 128), 1);
+    tm.tic(2);
+    if (r->store_dtype == 64)
+        snapshot_kernel<double><<<sg, 128, 0, stream>>>(m->n_params, m->n_groups, partial ? 1 : 0, s->n_chains, s->stride,
+                                                        s->theta, s->hyper, (double*)r->store + (size_t)row * ncol * S);
+    else
+        snapshot_kernel<float><<<sg, 128, 0, stream>>>(m->n_params, m->n_groups, partial ? 1 : 0, s->n_chains, s->stride,
+                                                       s->theta, s->hyper, (float*)r->store + (size_t)row * ncol * S);
+    tm.toc();
+    if (r->loglik_store) {
+        const int rc = launch_pointwise(ks, m, s, r->loglik_store + (size_t)row * (size_t)m->n_obs * S, stream);
+        if (rc) return rc;
+    }
+    ++row;
+    return MCMCN_OK;
+}
+
 // Complete pooling with the observations split into small groups (mcmcn_model.split): per sweep
-// propose -> eval over the small groups -> decide.  Same iteration bookkeeping as mcmcn_run.
-static int run_complete_split(const mcmcn_model* m, const mcmcn_state* s, const mcmcn_run_args* r, cudaStream_t stream) {
+// propose -> eval over the small groups -> decide.  `mks` is the kernel set of the model m itself
+// (pointwise log-likelihood of the retained rows).
+static int run_complete_split(const KernelSet* mks, const mcmcn_model* m, const mcmcn_state* s, const mcmcn_run_args* r,
+                              cudaStream_t stream) {
     const mcmcn_model* e = m->split;
     const KernelSet* ks = nullptr;
     int rc = validate(e, s, &ks);
@@ -263,29 +337,22 @@ static int run_complete_split(const mcmcn_model* m, const mcmcn_state* s, const 
     c.chain_id0 = s->chain_id0; c.seed = r->seed;
     c.theta = s->theta; c.scale = s->scale; c.counts = s->counts; c.ll = s->ll; c.lprior = s->lprior;
     c.cand = cand; c.part = part; c.park = park;
-    const size_t per_iter = (size_t)P * S;
-    long long last_tune = 0;
-    if (r->burn > 0) last_tune = ((long long)(r->burn - 1) / r->tune_interval) * r->tune_interval;
+    const size_t per_iter = (size_t)P * S;                              // the one group of complete pooling
     int64_t row = r->store_row0;
+    KernelTimer tm = {r->timing, stream, false};                        // launch counts only
     const unsigned nb = (unsigned)((S + 127) / 128);
     for (int it = 0; it < r->n_iter; ++it) {
         const long long i = r->iter0 + it;
+        const IterFlags f = iter_flags(r, i);
         c.iter = i;
-        c.tune = (i != 0 && i < r->burn && (i % r->tune_interval) == 0) ? 1 : 0;
-        c.count = (i <= last_tune) ? 1 : 0;
-        c.tape_z = r->tape_z ? r->tape_z + it * per_iter : nullptr;
-        c.tape_u = r->tape_u ? r->tape_u + it * per_iter : nullptr;
-        c.tape_acc = r->tape_accept ? r->tape_accept + it * per_iter : nullptr;
-        c.tr_ll = r->trace_ll ? r->trace_ll + it * per_iter : nullptr;
-        c.tr_lp = r->trace_lp ? r->trace_lp + it * per_iter : nullptr;
-        c.tr_diff = r->trace_diff ? r->trace_diff + it * per_iter : nullptr;
-        c.tr_acc = r->trace_accept ? r->trace_accept + it * per_iter : nullptr;
-        if (c.tr_ll && !(c.tr_lp && c.tr_diff && c.tr_acc)) { set_error("trace arrays go together"); return MCMCN_ERR_INVALID; }
+        c.tune = f.tune;
+        c.count = f.count;
+        c.tp = iter_tapes(r, it, per_iter);
         for (int p = 0; p < P; ++p) {                                   // StepMethod.step, :594-597
             c.p = p;
             c.prior = m->prior[p];
             if (p == 0) complete_propose_kernel<<<nb, 128, 0, stream>>>(c);       // later names: proposed by the decide launch before
-            if (r->timing) r->timing[3] += 1.0;
+            tm.tic(0);
             if (etc) {
                 void* args[] = {&ta};
                 CK(cudaLaunchKernel((const void*)tfn, tg.grid, tg.block, args, tg.smem, stream));
@@ -295,23 +362,10 @@ static int run_complete_split(const mcmcn_model* m, const mcmcn_state* s, const 
             c.propose_next = p + 1 < P ? 1 : 0;
             c.prior_next = m->prior[p + 1 < P ? p + 1 : p];
             complete_decide_kernel<<<(unsigned)(S / 32), dim3(32, 32, 1), 0, stream>>>(c);
+            tm.toc();
         }
-        if (r->store && i >= r->burn && (i % r->thin) == 0) {
-            if (row >= r->store_rows) { set_error("sample store overflow at row %lld", (long long)row); return MCMCN_ERR_INVALID; }
-            const dim3 sg((unsigned)((P + MCMCN_SNAP_COLS - 1) / MCMCN_SNAP_COLS), (unsigned)((s->n_chains + 127) / 128), 1);
-            if (r->timing) r->timing[5] += 1.0;
-            if (r->store_dtype == 64)
-                snapshot_kernel<double><<<sg, 128, 0, stream>>>(P, 1, 0, s->n_chains, S, s->theta, s->hyper, (double*)r->store + (size_t)row * P * S);
-            else
-                snapshot_kernel<float><<<sg, 128, 0, stream>>>(P, 1, 0, s->n_chains, S, s->theta, s->hyper, (float*)r->store + (size_t)row * P * S);
-            if (r->loglik_store) {
-                const KernelSet* mks = nullptr;
-                int prc = validate(m, s, &mks);
-                if (!prc) prc = launch_pointwise(mks, m, s, r->loglik_store + (size_t)row * (size_t)m->n_obs * S, stream);
-                if (prc) return prc;
-            }
-            ++row;
-        }
+        rc = write_retained_row(mks, m, s, r, i, row, tm, stream);
+        if (rc) return rc;
     }
     CK(cudaGetLastError());
     return MCMCN_OK;
@@ -341,13 +395,14 @@ int mcmcn_run(const mcmcn_model* m, const mcmcn_state* s, const mcmcn_run_args* 
     if (r->loglik_store && !r->store) { set_error("loglik_store goes with store (same rows)"); return MCMCN_ERR_INVALID; }
     if (r->tune_interval > 65535) { set_error("tune_interval %d: the accept / reject counters since the last tune are 16 bits each", r->tune_interval); return MCMCN_ERR_INVALID; }
     if ((r->tape_z == nullptr) != (r->tape_u == nullptr)) { set_error("tape_z and tape_u go together"); return MCMCN_ERR_INVALID; }
+    if (r->trace_ll && !(r->trace_lp && r->trace_diff && r->trace_accept)) { set_error("trace arrays go together"); return MCMCN_ERR_INVALID; }
     const bool partial = m->pooling == MCMCN_POOL_PARTIAL;
     if (partial && !s->hyper) { set_error("partial pooling needs state.hyper"); return MCMCN_ERR_INVALID; }
     if (!partial && !s->lprior) { set_error("fixed priors need state.lprior"); return MCMCN_ERR_INVALID; }
     if (partial && m->n_groups < 2) { set_error("partial pooling needs at least 2 groups"); return MCMCN_ERR_INVALID; }
     if (partial && r->tape_z && (!r->tape_zmu || !r->tape_qsig)) { set_error("replay of partial pooling needs tape_zmu/tape_qsig"); return MCMCN_ERR_INVALID; }
     cudaStream_t stream = (cudaStream_t)stream_;
-    if (m->pooling == MCMCN_POOL_COMPLETE && m->split && !getenv("MCMCN_NO_SPLIT")) return run_complete_split(m, s, r, stream);
+    if (m->pooling == MCMCN_POOL_COMPLETE && m->split && !getenv("MCMCN_NO_SPLIT")) return run_complete_split(ks, m, s, r, stream);
 
     SweepArgs a;
     fill_args(a, ks, m, s);
@@ -380,47 +435,24 @@ int mcmcn_run(const mcmcn_model* m, const mcmcn_state* s, const mcmcn_run_args* 
     const size_t S = (size_t)s->stride;
     const size_t per_iter = (size_t)m->n_params * m->n_groups * S;
     const size_t per_iter_h = (size_t)m->n_params * S;
-    const int ncol = m->n_params * (m->n_groups + (partial ? 2 : 0));
-    // counters are only ever read by tune(), which stops at the last multiple of tune_interval below burn
-    long long last_tune = 0;
-    if (r->burn > 0) last_tune = ((long long)(r->burn - 1) / r->tune_interval) * r->tune_interval;
     int64_t row = r->store_row0;
-
-    // optional per-kernel timing: launches are always counted; every 8th iteration's launches are
-    // bracketed by event pairs that mcmcn_timing_collect() reads later, so the call stays asynchronous
-    bool sample_it = false;
-    auto tic = [&](int kind) {
-        if (!r->timing) return;
-        r->timing[3 + kind] += 1.0;
-        if (!sample_it) return;
-        Stamp st; st.kind = kind; st.out = r->timing;
-        cudaEventCreate(&st.e0); cudaEventCreate(&st.e1);
-        cudaEventRecord(st.e0, stream);
-        g_stamps.push_back(st);
-    };
-    auto toc = [&]() { if (r->timing && sample_it) cudaEventRecord(g_stamps.back().e1, stream); };
+    KernelTimer tm = {r->timing, stream, false};
 
     for (int it = 0; it < r->n_iter; ++it) {
         const long long i = r->iter0 + it;
-        sample_it = (i & 7) == 0;
+        const IterFlags f = iter_flags(r, i);
+        tm.sampled = (i & 7) == 0;                                     // every 8th iteration's launches are timed
         a.iter = i;
         a.seed = r->seed;
-        a.tune = (i != 0 && i < r->burn && (i % r->tune_interval) == 0) ? 1 : 0;
-        a.count = (i <= last_tune) ? 1 : 0;
+        a.tune = f.tune;
+        a.count = f.count;
         a.use_override = (it == 0 && r->use_lprior_override && partial) ? 1 : 0;
-        a.tape_z = r->tape_z ? r->tape_z + it * per_iter : nullptr;
-        a.tape_u = r->tape_u ? r->tape_u + it * per_iter : nullptr;
-        a.tape_acc = r->tape_accept ? r->tape_accept + it * per_iter : nullptr;
-        a.tr_ll = r->trace_ll ? r->trace_ll + it * per_iter : nullptr;
-        a.tr_lp = r->trace_lp ? r->trace_lp + it * per_iter : nullptr;
-        a.tr_diff = r->trace_diff ? r->trace_diff + it * per_iter : nullptr;
-        a.tr_acc = r->trace_accept ? r->trace_accept + it * per_iter : nullptr;
-        if (a.tr_ll && !(a.tr_lp && a.tr_diff && a.tr_acc)) { set_error("trace arrays go together"); return MCMCN_ERR_INVALID; }
+        a.tp = iter_tapes(r, it, per_iter);
         const int fidx = (partial ? MCMCN_F_PARTIAL : 0) | (a.count ? MCMCN_F_COUNT : 0);
         const sweep_fn fn = (fast && !a.use_override) ? fast_fn[fidx] : general;
-        tic(0);
+        tm.tic(0);
         CK(launch_sweep(fn, g.grid, g.block, g.smem, stream, a));
-        toc();
+        tm.toc();
 
         if (partial) {
             HyperArgs h;
@@ -430,7 +462,7 @@ int mcmcn_run(const mcmcn_model* m, const mcmcn_state* s, const mcmcn_run_args* 
             h.tape_zmu = r->tape_zmu ? r->tape_zmu + it * per_iter_h : nullptr;
             h.tape_qsig = r->tape_qsig ? r->tape_qsig + it * per_iter_h : nullptr;
             const dim3 hg((unsigned)((s->n_chains + 31) / 32), (unsigned)m->n_params, 1);
-            tic(1);
+            tm.tic(1);
             if (m->n_groups >= 512 && !getenv("MCMCN_HYPER_TWO_PASS"))
             {
                 // the widest block row that still leaves about two blocks per SM (the sums do not depend on the shape)
@@ -445,26 +477,10 @@ int mcmcn_run(const mcmcn_model* m, const mcmcn_state* s, const mcmcn_run_args* 
             else if (m->n_groups >= 512) hyper_kernel<32><<<hg, dim3(32, 32, 1), 0, stream>>>(h);
             else if (m->n_groups >= 64) hyper_kernel<8><<<hg, dim3(32, 8, 1), 0, stream>>>(h);
             else hyper_kernel<1><<<hg, dim3(32, 1, 1), 0, stream>>>(h);
-            toc();
+            tm.toc();
         }
-
-        if (r->store && i >= r->burn && (i % r->thin) == 0) {
-            if (row >= r->store_rows) { set_error("sample store overflow at row %lld", (long long)row); return MCMCN_ERR_INVALID; }
-            const dim3 sg((unsigned)((ncol + MCMCN_SNAP_COLS - 1) / MCMCN_SNAP_COLS), (unsigned)((s->n_chains + 127) / 128), 1);
-            tic(2);
-            if (r->store_dtype == 64)
-                snapshot_kernel<double><<<sg, 128, 0, stream>>>(m->n_params, m->n_groups, partial ? 1 : 0, s->n_chains, s->stride,
-                                                                s->theta, s->hyper, (double*)r->store + (size_t)row * ncol * S);
-            else
-                snapshot_kernel<float><<<sg, 128, 0, stream>>>(m->n_params, m->n_groups, partial ? 1 : 0, s->n_chains, s->stride,
-                                                               s->theta, s->hyper, (float*)r->store + (size_t)row * ncol * S);
-            toc();
-            if (r->loglik_store) {                                     // Sampler._printLogLikelihood, :890-891, :907-909
-                rc = launch_pointwise(ks, m, s, r->loglik_store + (size_t)row * (size_t)m->n_obs * S, stream);
-                if (rc) return rc;
-            }
-            ++row;
-        }
+        rc = write_retained_row(ks, m, s, r, i, row, tm, stream);
+        if (rc) return rc;
     }
     CK(cudaGetLastError());
     return MCMCN_OK;
@@ -533,19 +549,16 @@ namespace mcmcn {
 __global__ void debug_draws_kernel(int kind, long long n, unsigned long long seed, double a, double* out) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    // chain id = i, iteration 7, name/group index 3: any fixed counter will do, the key carries i
-    const uint4 r = philox_draw(i, seed, 7, MCMCN_STREAM_SWEEP, 3u, 1u);
+    // chain id = i, iteration 7, name/group index 3 (sweep 0 of group 3, G = 1): any fixed counter will do, the key carries i
+    const SweepDraws d = sweep_draws(i, seed, 7, 0, 1, 3);
     switch (kind) {
-        case MCMCN_DRAW_SWEEP_NORMALS: {          // both Box-Muller branches of the sweep draw: out[2i], out[2i+1]
-            float zc, zs;
-            normal_pair_from(r.x, r.y, zc, zs);
-            out[2 * i] = (double)zc;
-            out[2 * i + 1] = (double)zs;
+        case MCMCN_DRAW_SWEEP_NORMALS:            // both Box-Muller branches of the sweep draw: out[2i], out[2i+1]
+            out[2 * i] = (double)d.z0;
+            out[2 * i + 1] = (double)d.z1;
             break;
-        }
         case MCMCN_DRAW_SWEEP_UNIFORMS:           // the two accept uniforms of the sweep draw
-            out[2 * i] = uniform_from32(r.z);
-            out[2 * i + 1] = uniform_from32(r.w);
+            out[2 * i] = uniform_from32(d.u0);
+            out[2 * i + 1] = uniform_from32(d.u1);
             break;
         case MCMCN_DRAW_HYPER_NORMAL: {           // the mu draw of the Gibbs update
             const uint4 h = philox_draw(i, seed, 7, MCMCN_STREAM_HYPER, 3u, 0u);
@@ -555,9 +568,11 @@ __global__ void debug_draws_kernel(int kind, long long n, unsigned long long see
         case MCMCN_DRAW_UNIT_INVGAMMA:            // the sigma2 draw of the Gibbs update, unit scale
             out[i] = 1.0 / gamma_draw(a, i, seed, 7, 3u);
             break;
-        case MCMCN_DRAW_UNIFORM53:
+        case MCMCN_DRAW_UNIFORM53: {
+            const uint4 r = philox_draw(i, seed, 7, MCMCN_STREAM_SWEEP, 3u, 1u);
             out[i] = uniform_from(r.x, r.y);
             break;
+        }
         default:
             out[i] = __longlong_as_double(0x7ff8000000000000LL);
     }

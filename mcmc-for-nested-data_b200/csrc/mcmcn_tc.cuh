@@ -218,9 +218,7 @@ struct TcInputs {
     unsigned cnt;                   // burn-in: accepted | rejected << 16 since the last tune, fetched with the rest (not after the decision)
 };
 
-// One Philox4x32-10 call serves two consecutive sweeps: Box-Muller turns words 0-1 into two
-// standard normals (cosine and sine branch), words 2 and 3 give one 32-bit uniform each,
-// (w + 0.5) * 2^-32 in (0, 1).  `stash` carries the second pair to the odd sweep.
+// The odd sweep's (z, u) of sweep_draws, carried over from the even sweep.
 struct TcStash { double z, u; };
 
 // `at` = element index of (name p, group g, this chain) in the [P][G][S] arrays, `hy` = p * S + chain
@@ -231,7 +229,6 @@ __device__ __forceinline__ void tc_fetch_state(TcInputs& o, const SweepArgs& a, 
                                                bool partial, bool override_lp, bool count = false) {
     const int P = a.P;
     o.cnt = count ? a.counts[at] : 0u;
-    const size_t PS = (size_t)P * (size_t)a.S;
     o.cur = a.theta[at];
     o.sc = a.scale[at];
     o.h_mu = o.h_lsd = o.h_isd = o.lp_cur = 0.0;
@@ -249,16 +246,14 @@ template <bool GENERAL>
 __device__ __forceinline__ void tc_fetch_random(TcInputs& o, const SweepArgs& a, int p, int g, int chl, size_t at, bool replay,
                                                 TcStash& stash) {
     if (GENERAL && replay) {
-        o.z = a.tape_z[at];
-        o.u = a.tape_u[at];
+        o.z = a.tp.tape_z[at];
+        o.u = a.tp.tape_u[at];
     } else if ((p & 1) == 0) {
-        const uint4 rnd = philox_draw(a.chain_id0 + chl, a.seed, a.iter, MCMCN_STREAM_SWEEP, (unsigned)((p >> 1) * a.G + g), 1u);
-        float zc, zs;
-        normal_pair_from(rnd.x, rnd.y, zc, zs);
-        o.z = (double)zc;
-        stash.z = (double)zs;
-        o.u = uniform_from32(rnd.z);
-        stash.u = uniform_from32(rnd.w);
+        const SweepDraws d = sweep_draws(a.chain_id0 + chl, a.seed, a.iter, p, a.G, g);
+        o.z = (double)d.z0;
+        stash.z = (double)d.z1;
+        o.u = uniform_from32(d.u0);
+        stash.u = uniform_from32(d.u1);
     } else {
         o.z = stash.z;
         o.u = stash.u;
@@ -296,6 +291,48 @@ __device__ __forceinline__ bool tc_rendezvous_issuer() {
     return issuer;
 }
 
+// CTA prologue of the tcgen05 kernels, called by every thread: three mbarriers ([0..1] TMA stage full, [2]
+// accumulator full), the constant A operand of the ne MMA, and the CTA's MCMCN_TC_COLS tensor-memory columns.
+struct TcCta {
+    unsigned ones, stage0;        // shared-memory addresses of the ones operand and of TMA stage 0 (1024-byte aligned)
+    unsigned tbase, tlane;        // the CTA's first TMEM column; the same with this warp's lane field (32 * warp)
+    unsigned mb_tma0, mb_mma;     // mbarrier of stage 0 (stage s: + 8 s) and of the accumulator
+};
+__device__ __forceinline__ TcCta tc_cta_begin(unsigned char* smem_raw, unsigned long long (&mbar_s)[3], unsigned* tmem_base_s) {
+    const int tid = threadIdx.x, warp = tid >> 5;
+    TcCta t;
+    t.ones = (smem_u32(smem_raw) + 1023u) & ~1023u;
+    t.stage0 = t.ones + MCMCN_TC_ONES_BYTES;
+    if (tid == 0) {
+#pragma unroll
+        for (int i = 0; i < 3; ++i) mbar_init(smem_u32(&mbar_s[i]), 1);
+    }
+    {   // constant A operand of the ne MMA: every row (1, 1, 1, 0 | 0, 0, 0, 0), K-major core matrices
+        for (int i = tid; i < MCMCN_TC_ONES_BYTES / 16; i += MCMCN_TC_THREADS) {
+            const float one = ((i >> 3) & 1) == 0 ? 1.0f : 0.0f;      // 8 rows x 16 bytes per K half
+            asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(t.ones + 16u * i), "f"(one), "f"(one), "f"(one), "f"(0.0f) : "memory");
+        }
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy writes -> tensor core reads
+    }
+    if (warp == 0) tmem_alloc(tmem_base_s, MCMCN_TC_COLS);
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    t.tbase = *tmem_base_s;
+    t.tlane = t.tbase + ((unsigned)warp << 21);
+    t.mb_tma0 = smem_u32(&mbar_s[0]);
+    t.mb_mma = smem_u32(&mbar_s[2]);
+    asm volatile("" : "+r"(t.mb_tma0), "+r"(t.mb_mma));              // held in registers (else rebuilt from SR_CgaCtaId at every wait)
+    return t;
+}
+// CTA epilogue: every tensor-memory access of the CTA is done before warp 0 frees its columns
+__device__ __forceinline__ void tc_cta_end(const TcCta& t) {
+    tmem_wait_st();
+    tc_fence_before();
+    __syncthreads();
+    if ((threadIdx.x >> 5) == 0) tmem_free(t.tbase, MCMCN_TC_COLS);
+}
+
 // grid = (group ranges, chain blocks of 128); block = 128 threads; dynamic shared memory =
 // the constant ones operand + a.tc_stages (2, or 1 for big groups) stages of a.tc_stage_bytes (1024-byte aligned).
 // UNIFORM208: every group of the model pads to 208 observations (193-208, BASELINE config 3's 200): the
@@ -311,9 +348,9 @@ __global__ void __launch_bounds__(MCMCN_TC_THREADS, 4) sweep_tc_kernel(const Swe
     constexpr bool GENERAL = F < 0;
     const bool partial = GENERAL ? (a.partial != 0) : ((F & MCMCN_F_PARTIAL) != 0);
     const bool count = GENERAL ? (a.count != 0) : ((F & MCMCN_F_COUNT) != 0);
-    const bool replay = GENERAL && a.tape_z != nullptr;
-    const bool trace = GENERAL && a.tr_ll != nullptr;
-    const bool forced = GENERAL && a.tape_acc != nullptr;
+    const bool replay = GENERAL && a.tp.tape_z != nullptr;
+    const bool trace = GENERAL && a.tp.tr_ll != nullptr;
+    const bool forced = GENERAL && a.tp.tape_acc != nullptr;
     const bool override_lp = GENERAL && a.use_override != 0;
     const int P = a.P, K = a.P - 1;
 
@@ -325,39 +362,16 @@ __global__ void __launch_bounds__(MCMCN_TC_THREADS, 4) sweep_tc_kernel(const Swe
     const int g0 = (int)(((long long)a.G * blockIdx.x) / nr), g1 = (int)(((long long)a.G * (blockIdx.x + 1)) / nr);
     if (g0 >= g1) return;
 
-    const int tid = threadIdx.x, warp = tid >> 5;
-    const unsigned ones = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    const unsigned stage0 = ones + MCMCN_TC_ONES_BYTES;
-    if (tid == 0) {
-#pragma unroll
-        for (int i = 0; i < 3; ++i) mbar_init(smem_u32(&mbar_s[i]), 1);
-    }
-    {   // constant A operand of the ne MMA: every row (1, 1, 1, 0 | 0, 0, 0, 0), K-major core matrices
-        const float4 lo4 = make_float4(1.0f, 1.0f, 1.0f, 0.0f), z4 = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
-        for (int i = tid; i < MCMCN_TC_ONES_BYTES / 16; i += MCMCN_TC_THREADS) {
-            const bool first_half = ((i >> 3) & 1) == 0;               // 8 rows x 16 bytes per K half
-            asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(ones + 16u * i), "f"(first_half ? lo4.x : z4.x),
-                         "f"(first_half ? lo4.y : z4.y), "f"(first_half ? lo4.z : z4.z), "f"(z4.w) : "memory");
-        }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy writes -> tensor core reads
-    }
-    if (warp == 0) tmem_alloc(&tmem_base_s, MCMCN_TC_COLS);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const unsigned tbase = tmem_base_s;
-    const unsigned tlane = tbase + ((unsigned)warp << 21);             // lane field = 32 * warp
-    unsigned mb_tma0 = smem_u32(&mbar_s[0]), mb_mma = smem_u32(&mbar_s[2]);
-    asm volatile("" : "+r"(mb_tma0), "+r"(mb_mma));                    // held in registers (else rebuilt from SR_CgaCtaId at every wait)
-
+    const int tid = threadIdx.x;
+    const TcCta t = tc_cta_begin(smem_raw, mbar_s, &tmem_base_s);
     const float* tc = reinterpret_cast<const float*>(a.tc_data);
     auto stage_group = [&](int s, int g) {                             // thread 0 only
         const long long e0 = a.tc_group_off[g], e1 = a.tc_group_off[g + 1];
         const unsigned bytes = (unsigned)((e1 - e0) * 4);
         MCMCN_CHECK(s >= 0 && s < a.tc_stages && g >= g0 && g < g1);
         MCMCN_CHECK(bytes > 0 && (bytes & 15u) == 0u && (int)bytes <= a.tc_stage_bytes && ((e0 * 4) & 15) == 0);   // TMA extent
-        mbar_expect_tx(mb_tma0 + 8u * s, bytes);
-        tma_bulk_g2s(stage0 + (unsigned)s * (unsigned)a.tc_stage_bytes, tc + e0, bytes, mb_tma0 + 8u * s);
+        mbar_expect_tx(t.mb_tma0 + 8u * s, bytes);
+        tma_bulk_g2s(t.stage0 + (unsigned)s * (unsigned)a.tc_stage_bytes, tc + e0, bytes, t.mb_tma0 + 8u * s);
     };
     if (tid == 0) {
         stage_group(0, g0);
@@ -378,9 +392,9 @@ __global__ void __launch_bounds__(MCMCN_TC_THREADS, 4) sweep_tc_kernel(const Swe
         const int np = max(16, (R + 15) & ~15);                        // padded observation count of the block
         const int nchunks = (np + CH - 1) / CH;
         MCMCN_CHECK(R >= 0 && np * 32 * (2 * KB + 1) == (int)((a.tc_group_off[g + 1] - a.tc_group_off[g]) * 4));   // 2 KB + 1 slabs of [np][8] floats
-        MCMCN_CHECK(np * 32 * (2 * KB + 1) <= a.tc_stage_bytes && (tbase & 0xFFFFu) + MCMCN_TC_COLS <= 512u);
+        MCMCN_CHECK(np * 32 * (2 * KB + 1) <= a.tc_stage_bytes && (t.tbase & 0xFFFFu) + MCMCN_TC_COLS <= 512u);
         MCMCN_CHECK(K >= 1 && K <= 8 * KB);
-        const unsigned stage = stage0 + (unsigned)s * (unsigned)a.tc_stage_bytes;
+        const unsigned stage = t.stage0 + (unsigned)s * (unsigned)a.tc_stage_bytes;
         const double* bbar = a.obj_const + (size_t)g * K;
 
         const size_t GS = (size_t)a.G * S;
@@ -397,7 +411,7 @@ __global__ void __launch_bounds__(MCMCN_TC_THREADS, 4) sweep_tc_kernel(const Swe
         // The proposal of a sweep and its centred FP32 value are formed at the end of the sweep before
         // (here: for sweep 0), so that column p (the value kept) and column p + 1 (the next proposal) of
         // the A operand go out in one two-column store.
-        double prop = __dadd_rn(in.cur, __dmul_rn(in.sc, in.z));      // numpy.random.normal(value, sd), :304-306
+        double prop = propose(in.cur, in.sc, in.z);
         float wcur = (float)__dsub_rn(in.cur, in.bbar), wprop = (float)__dsub_rn(prop, in.bbar);
         {   // A operand of the current state: centred coefficients (FP32), split hi / lo, 8 columns per K block
             const double* tk = tg;
@@ -412,14 +426,14 @@ __global__ void __launch_bounds__(MCMCN_TC_THREADS, 4) sweep_tc_kernel(const Swe
                     hi[j] = tf32_rn(b);
                     lo[j] = tf32_rn(b - __uint_as_float(hi[j]));
                 }
-                tmem_st8(tlane + M::A_HI + 8 * kb, hi);
-                tmem_st8(tlane + M::A_LO + 8 * kb, lo);
+                tmem_st8(t.tlane + M::A_HI + 8 * kb, hi);
+                tmem_st8(t.tlane + M::A_LO + 8 * kb, lo);
             }
         }
         double aux_m, aux_r;                                           // LinReg::Aux of the current sigma
         tc_sigma_terms(tg[(size_t)K * GS], R, aux_m, aux_r);
         double ll_cur = a.ll[at];
-        mbar_wait(mb_tma0 + 8u * s, (tma_phase >> s) & 1u);
+        mbar_wait(t.mb_tma0 + 8u * s, (tma_phase >> s) & 1u);
         tma_phase ^= 1u << s;
 
 #pragma unroll 1
@@ -443,7 +457,7 @@ __global__ void __launch_bounds__(MCMCN_TC_THREADS, 4) sweep_tc_kernel(const Swe
             const float wcur_now = wcur, wprop_now = wprop;            // this sweep's; wcur / wprop move on to the next below
             if (is_sigma) tc_sigma_terms(prop, R, m_prop, r_prop);     // LinReg::aux of the proposed sigma
             tmem_wait_st();
-            if (tc_rendezvous_issuer()) tc_issue_chunk<KB>(tbase, stage, ones, np, 0, mb_mma);
+            if (tc_rendezvous_issuer()) tc_issue_chunk<KB>(t.tbase, stage, t.ones, np, 0, t.mb_mma);
             // while the tensor core works: state and random numbers of the next sweep.  (Drawing the
             // random numbers inside the read-back code instead, to fill its tensor-memory latency, cost
             // registers and measured 8 % slower.)
@@ -455,55 +469,44 @@ __global__ void __launch_bounds__(MCMCN_TC_THREADS, 4) sweep_tc_kernel(const Swe
             double acc = 0.0;
             if (UNIFORM208 && np == 208) {                             // 112 + 96 observations (C3's groups): straight line, one fold
                 f32x2 sq[4] = {0ull, 0ull, 0ull, 0ull};
-                mbar_wait(mb_mma, mma_phase);
+                mbar_wait(t.mb_mma, mma_phase);
                 tc_fence_after();
-                tc_accumulate_fixed<7>(tlane + MCMCN_TC_D, sq);
-                if (tc_rendezvous_issuer()) tc_issue_chunk<KB>(tbase, stage, ones, np, 1, mb_mma);
-                mbar_wait(mb_mma, mma_phase ^ 1u);
+                tc_accumulate_fixed<7>(t.tlane + MCMCN_TC_D, sq);
+                if (tc_rendezvous_issuer()) tc_issue_chunk<KB>(t.tbase, stage, t.ones, np, 1, t.mb_mma);
+                mbar_wait(t.mb_mma, mma_phase ^ 1u);
                 tc_fence_after();
-                tc_accumulate_fixed<6>(tlane + MCMCN_TC_D, sq);
+                tc_accumulate_fixed<6>(t.tlane + MCMCN_TC_D, sq);
                 acc = (double)((sum2(sq[0]) + sum2(sq[1])) + (sum2(sq[2]) + sum2(sq[3])));
             } else if (!UNIFORM208 && KB == 1 && nchunks == 2) {       // any group of 113-224 observations: the same, second chunk looped
                 f32x2 sq[4] = {0ull, 0ull, 0ull, 0ull};
-                mbar_wait(mb_mma, mma_phase);
+                mbar_wait(t.mb_mma, mma_phase);
                 tc_fence_after();
-                tc_accumulate_fixed<7>(tlane + MCMCN_TC_D, sq);
-                if (tc_rendezvous_issuer()) tc_issue_chunk<KB>(tbase, stage, ones, np, 1, mb_mma);
-                mbar_wait(mb_mma, mma_phase ^ 1u);
+                tc_accumulate_fixed<7>(t.tlane + MCMCN_TC_D, sq);
+                if (tc_rendezvous_issuer()) tc_issue_chunk<KB>(t.tbase, stage, t.ones, np, 1, t.mb_mma);
+                mbar_wait(t.mb_mma, mma_phase ^ 1u);
                 tc_fence_after();
-                tc_accumulate_any(tlane + MCMCN_TC_D, (np - CH) >> 4, sq);
+                tc_accumulate_any(t.tlane + MCMCN_TC_D, (np - CH) >> 4, sq);
                 acc = (double)((sum2(sq[0]) + sum2(sq[1])) + (sum2(sq[2]) + sum2(sq[3])));
             } else
             for (int c = 0; c < nchunks; ++c) {
-                mbar_wait(mb_mma, mma_phase);
+                mbar_wait(t.mb_mma, mma_phase);
                 mma_phase ^= 1u;
                 tc_fence_after();
                 const int nc = min(CH, np - c * CH);
-                acc += tc_sum_squares(tlane + MCMCN_TC_D, nc >> 4);
+                acc += tc_sum_squares(t.tlane + MCMCN_TC_D, nc >> 4);
                 if (c + 1 < nchunks) {                                 // the accumulator is free once every lane has read it
-                    if (tc_rendezvous_issuer()) tc_issue_chunk<KB>(tbase, stage, ones, np, c + 1, mb_mma);
+                    if (tc_rendezvous_issuer()) tc_issue_chunk<KB>(t.tbase, stage, t.ones, np, c + 1, t.mb_mma);
                 }
             }
 
-            // Parameter.step decision tree, :334-367
             const double llp = acc * m_prop - r_prop;
             const double post_prop = lp_prop + llp;
             const double post_cur = lp_cur + ll_cur;
             const double diff = post_prop - post_cur;
-            const bool b1 = !finite64(post_cur) && finite64(post_prop);
-            const bool test = finite64(llp) && finite64(diff);         // branches 4/5 draw the uniform
-            const int fast = log_u_vs_diff_fast(u, diff);
-            bool accept = b1 || (test && fast > 0);
-            if (!b1 && test && fast == 0) accept = log(u) < diff;      // rare: within 1e-6 of the threshold
-            if (GENERAL) {
-                if (trace && on) {
-                    a.tr_ll[at] = llp;
-                    a.tr_lp[at] = lp_prop;
-                    a.tr_diff[at] = diff;
-                    a.tr_acc[at] = accept ? 1 : 0;
-                }
-                if (forced) accept = a.tape_acc[at] != 0;
-            }
+            bool exact;
+            bool accept = decide_fast(post_cur, post_prop, llp, diff, u, exact);
+            if (exact) accept = decide_exact(u, diff);                 // rare: within 1e-6 of the threshold
+            if (GENERAL) accept = trace_and_force(a.tp, at, trace && on, forced, llp, lp_prop, diff, accept);
             if (accept) {                                              // :369-378, :608-610
                 if (on) {
                     a.theta[at] = prop;
@@ -516,51 +519,26 @@ __global__ void __launch_bounds__(MCMCN_TC_THREADS, 4) sweep_tc_kernel(const Swe
             if (!is_sigma) {                                           // column p <- the value the chain keeps, column p + 1 <- the next proposal
                 const float wkeep = accept ? wprop_now : wcur_now;
                 const unsigned h = tf32_rn(wkeep), l = tf32_rn(wkeep - __uint_as_float(h));
-                prop = __dadd_rn(in.cur, __dmul_rn(in.sc, in.z));      // `in` holds sweep p + 1 by now
+                prop = propose(in.cur, in.sc, in.z);                   // `in` holds sweep p + 1 by now
                 MCMCN_CHECK(p >= 0 && p < 8 * KB && p < K);                             // A-operand column
                 if (p + 1 < K) {
                     wcur = (float)__dsub_rn(in.cur, in.bbar);
                     wprop = (float)__dsub_rn(prop, in.bbar);
                     const unsigned nh = tf32_rn(wprop);
-                    tmem_st2(tlane + M::A_HI + p, h, nh);
-                    tmem_st2(tlane + M::A_LO + p, l, tf32_rn(wprop - __uint_as_float(nh)));
+                    tmem_st2(t.tlane + M::A_HI + p, h, nh);
+                    tmem_st2(t.tlane + M::A_LO + p, l, tf32_rn(wprop - __uint_as_float(nh)));
                 } else {                                               // the next sweep is sigma's: no column of its own
-                    tmem_st1(tlane + M::A_HI + p, h);
-                    tmem_st1(tlane + M::A_LO + p, l);
+                    tmem_st1(t.tlane + M::A_HI + p, h);
+                    tmem_st1(t.tlane + M::A_LO + p, l);
                 }
             }
-            if (count && on) {
-                unsigned cnt = cnt_now;
-                cnt += accept ? 1u : 0x10000u;
-                if (a.tune) {                                          // Parameter.tune, :385-437
-                    const unsigned na = cnt & 0xFFFFu, nrj = cnt >> 16;
-                    if (na + nrj) {
-                        const double sc = a.scale[at];
-                        const double rate = (double)na / (double)(na + nrj);
-                        double f = 1.0;
-                        if (rate < 0.001) f = 0.1;
-                        else if (rate < 0.05) f = 0.5;
-                        else if (rate < 0.2) f = 0.9;
-                        else if (rate > 0.95) f = 10.0;
-                        else if (rate > 0.75) f = 2.0;
-                        else if (rate > 0.5) f = 1.1;
-                        double ns = __dmul_rn(sc, f);
-                        if (ns == 0.0) ns = sc;
-                        a.scale[at] = ns;
-                        cnt = 0;
-                    }
-                }
-                a.counts[at] = cnt;
-            }
+            if (count && on) a.counts[at] = count_and_tune(cnt_now, accept, a.tune, a.scale + at);
         }
         if (on) a.ll[(size_t)g * S + chl] = ll_cur;
         // every MMA that read this stage has completed (all threads waited on its mbarrier)
         if (tid == 0 && g + a.tc_stages < g1) stage_group(s, g + a.tc_stages);
     }
-    tmem_wait_st();
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) tmem_free(tbase, MCMCN_TC_COLS);
+    tc_cta_end(t);
 }
 
 // ---------------------------------------------------------------- complete pooling: evaluation on the tensor core
@@ -583,37 +561,16 @@ __global__ void __launch_bounds__(MCMCN_TC_THREADS, 4) eval_tc_kernel(const Eval
 
     const int nr = gridDim.x;
     const int g0 = (int)(((long long)a.G * blockIdx.x) / nr), g1 = (int)(((long long)a.G * (blockIdx.x + 1)) / nr);
-    const int tid = threadIdx.x, warp = tid >> 5;
-    const unsigned ones = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    const unsigned stage0 = ones + MCMCN_TC_ONES_BYTES;
-    if (tid == 0) {
-#pragma unroll
-        for (int i = 0; i < 3; ++i) mbar_init(smem_u32(&mbar_s[i]), 1);
-    }
-    {   // constant A operand of the ne MMA: every row (1, 1, 1, 0 | 0, 0, 0, 0), K-major core matrices
-        for (int i = tid; i < MCMCN_TC_ONES_BYTES / 16; i += MCMCN_TC_THREADS) {
-            const float one = ((i >> 3) & 1) == 0 ? 1.0f : 0.0f;      // 8 rows x 16 bytes per K half
-            asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(ones + 16u * i), "f"(one), "f"(one), "f"(one), "f"(0.0f) : "memory");
-        }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    }
-    if (warp == 0) tmem_alloc(&tmem_base_s, MCMCN_TC_COLS);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const unsigned tbase = tmem_base_s;
-    const unsigned tlane = tbase + ((unsigned)warp << 21);
-    unsigned mb_tma0 = smem_u32(&mbar_s[0]), mb_mma = smem_u32(&mbar_s[2]);
-    asm volatile("" : "+r"(mb_tma0), "+r"(mb_mma));
-
+    const int tid = threadIdx.x;
+    const TcCta t = tc_cta_begin(smem_raw, mbar_s, &tmem_base_s);
     const float* tc = reinterpret_cast<const float*>(a.tc_data);
     auto stage_group = [&](int s, int g) {                             // thread 0 only
         const long long e0 = a.tc_group_off[g], e1 = a.tc_group_off[g + 1];
         const unsigned bytes = (unsigned)((e1 - e0) * 4);
         MCMCN_CHECK(s >= 0 && s < 2 && g >= g0 && g < g1);
         MCMCN_CHECK(bytes > 0 && (bytes & 15u) == 0u && (int)bytes <= a.tc_stage_bytes && ((e0 * 4) & 15) == 0);
-        mbar_expect_tx(mb_tma0 + 8u * s, bytes);
-        tma_bulk_g2s(stage0 + (unsigned)s * (unsigned)a.tc_stage_bytes, tc + e0, bytes, mb_tma0 + 8u * s);
+        mbar_expect_tx(t.mb_tma0 + 8u * s, bytes);
+        tma_bulk_g2s(t.stage0 + (unsigned)s * (unsigned)a.tc_stage_bytes, tc + e0, bytes, t.mb_tma0 + 8u * s);
     };
     if (tid == 0 && g0 < g1) {
         stage_group(0, g0);
@@ -636,8 +593,8 @@ __global__ void __launch_bounds__(MCMCN_TC_THREADS, 4) eval_tc_kernel(const Eval
                 hi[j] = tf32_rn(b);
                 lo[j] = tf32_rn(b - __uint_as_float(hi[j]));
             }
-            tmem_st8(tlane + M::A_HI + 8 * kb, hi);
-            tmem_st8(tlane + M::A_LO + 8 * kb, lo);
+            tmem_st8(t.tlane + M::A_HI + 8 * kb, hi);
+            tmem_st8(t.tlane + M::A_LO + 8 * kb, lo);
         }
     }
     double aux_m, aux_r1;                                              // -1/(2 sigma^2); log sigma + log sqrt(2 pi) (per observation)
@@ -652,28 +609,25 @@ __global__ void __launch_bounds__(MCMCN_TC_THREADS, 4) eval_tc_kernel(const Eval
         const int R = a.group_nobs[g];
         const int np = max(16, (R + 15) & ~15);
         const int nchunks = (np + CH - 1) / CH;
-        const unsigned stage = stage0 + (unsigned)s * (unsigned)a.tc_stage_bytes;
+        const unsigned stage = t.stage0 + (unsigned)s * (unsigned)a.tc_stage_bytes;
         MCMCN_CHECK(np * 32 * (2 * KB + 1) == (int)((a.tc_group_off[g + 1] - a.tc_group_off[g]) * 4));
         nobs += R;
-        mbar_wait(mb_tma0 + 8u * s, (tma_phase >> s) & 1u);
+        mbar_wait(t.mb_tma0 + 8u * s, (tma_phase >> s) & 1u);
         tma_phase ^= 1u << s;
         for (int c = 0; c < nchunks; ++c) {
             // every lane has read the accumulator of the chunk before (and, the first time, written its A operand)
-            if (tc_rendezvous_issuer()) tc_issue_chunk<KB>(tbase, stage, ones, np, c, mb_mma);
-            mbar_wait(mb_mma, mma_phase);
+            if (tc_rendezvous_issuer()) tc_issue_chunk<KB>(t.tbase, stage, t.ones, np, c, t.mb_mma);
+            mbar_wait(t.mb_mma, mma_phase);
             mma_phase ^= 1u;
             tc_fence_after();
             const int nc = min(CH, np - c * CH);
-            acc += tc_sum_squares(tlane + MCMCN_TC_D, nc >> 4);
+            acc += tc_sum_squares(t.tlane + MCMCN_TC_D, nc >> 4);
         }
         // every MMA that read this stage has completed (all threads waited on its mbarrier)
         if (tid == 0 && g + 2 < g1) stage_group(s, g + 2);
     }
     if (on) a.part[(size_t)blockIdx.x * S + ch] = acc * aux_m - (double)nobs * aux_r1;
-    tmem_wait_st();
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) tmem_free(tbase, MCMCN_TC_COLS);
+    tc_cta_end(t);
 }
 
 }  // namespace mcmcn

@@ -37,9 +37,14 @@ def burnThin(nIter, nSamples):
     return burn, thin
 
 
+def _retainedRange(lo, hi, burn, thin):
+    """Iterations i in [lo, hi) whose state Sampler._loop writes out: i >= burn and i % thin == 0 (:887)."""
+    return range(-(-max(lo, burn) // thin) * thin, hi, thin)
+
+
 def retainedIterations(nIter, burn, thin):
     """Iterations whose state Sampler._loop writes out (:887)."""
-    return [i for i in range(nIter) if i % thin == 0 and i >= burn]
+    return list(_retainedRange(0, nIter, burn, thin))
 
 
 def hostNormLogpdf(x, loc, scale):
@@ -134,8 +139,7 @@ PIN_SLOTS = int(os.environ.get("MCMCN_STORE_PIN_SLOTS", "2"))
 
 def retainedCount(lo, hi, burn, thin):
     """Number of iterations i in [lo, hi) that Sampler._loop retains (i >= burn and i % thin == 0, :887)."""
-    first = -(-max(lo, burn) // thin) * thin
-    return 0 if first >= hi else (hi - 1 - first) // thin + 1
+    return len(_retainedRange(lo, hi, burn, thin))
 
 
 class SampleStore(object):
@@ -699,8 +703,8 @@ class Engine(object):
             if room <= 0:
                 raise RuntimeError("sample store is full (%d rows)" % store.nRows)
             # last iteration of this piece = the room-th retained one from `cur` on (or the end of the call)
-            first = -(-max(cur, burn) // thin) * thin
-            stop = min(end, first + (room - 1) * thin + 1)
+            kept = _retainedRange(cur, end, burn, thin)
+            stop = kept[room - 1] + 1 if len(kept) >= room else end
             self._run(cur, stop - cur, burn, thin, store, None, False, tuneInterval, useLpriorOverride, timing)
             useLpriorOverride = None
             cur = stop
@@ -732,7 +736,7 @@ class Engine(object):
             a.store_dtype = 64 if store.dtype == torch.float64 else 32
             a.store_row0, a.store_rows = store.deviceRow()
             a.loglik_store = _ptr(store.logLik)
-            kept = [i for i in range(iter0, iter0 + nIter) if i % thin == 0 and i >= burn]
+            kept = list(_retainedRange(iter0, iter0 + nIter, burn, thin))
         if useLpriorOverride is None:
             useLpriorOverride = self.partial and self.lpriorStale and iter0 == 0
         a.use_lprior_override = 1 if useLpriorOverride else 0

@@ -1,6 +1,6 @@
 # Build a variant of one translation unit with extra -D flags into libmcmcn_<name>.so (same ABI; A/B with tools/ab.sh):
-#   bash tools/variant.sh <name> -DMCMCN_TC_X=1 ...                      (the tcgen05 step kernel, mcmcn_sets_tc.cu)
-#   UNIT=mcmcn_sets_logit bash tools/variant.sh <name> -DMCMCN_LOGIT_POLY_MASK=0 ...
+#   bash tools/variant.sh <name> -DMCMCN_DEBUG_BOUNDS                     (the tcgen05 step kernel, mcmcn_sets_tc.cu)
+#   UNIT=mcmcn_sets_logit bash tools/variant.sh <name> -DMY_SWITCH=1 ...   (a switch added to the source for the A/B)
 set -e
 name=$1; shift
 unit=${UNIT:-mcmcn_sets_tc}
