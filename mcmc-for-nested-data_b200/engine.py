@@ -19,6 +19,7 @@ import scipy.special
 import torch
 
 import mcmcn_native as nat
+from mcmcn_native import _hostThreads, _ptr
 from objectives import Objective
 
 _NORM_PDF_LOGC = numpy.log(numpy.sqrt(2 * numpy.pi))
@@ -117,24 +118,10 @@ def priorFromScipy(frozen):
     return pr
 
 
-def _ptr(t):
-    return ctypes.c_void_p(t.data_ptr()) if t is not None else None
-
-
-def _hostThreads(env):
-    """Host copy threads of this process: an even share of the cores among the ranks of this box, 2..8."""
-    share = (os.cpu_count() or 4) // max(1, int(os.environ.get("LOCAL_WORLD_SIZE", "1")))
-    return int(os.environ.get(env, max(2, min(8, share // 2))))
-
-
 WRITER_THREADS = _hostThreads("MCMCN_STORE_THREADS")
 # as many as writers: the file's pages are populated while the chains burn in and the writers have nothing to do (C3:
 # 37.8 GB in 2.9 s takes eight threads; with four the writers met unpopulated pages and the sampling phase waited)
 PREFAULT_THREADS = int(os.environ.get("MCMCN_PREFAULT_THREADS", WRITER_THREADS))
-# pinned staging chunks of the streamed sample store (the device ring stays at two chunks).  Two: measured at config 3
-# (profiles/experiments/r2_store_pin_slots_ab.log), 4 and 6 slots leave the sampling loop where it is or slower (5.96-5.98 s
-# against 6.06-6.13 and 6.47): the launching thread's wait for a slot is only its run-ahead being throttled, not device idle time
-PIN_SLOTS = int(os.environ.get("MCMCN_STORE_PIN_SLOTS", "2"))
 
 
 def retainedCount(lo, hi, burn, thin):
@@ -152,10 +139,11 @@ class SampleStore(object):
         chains have filled one chunk it is copied to pinned host memory on a side stream while they
         fill the other, and then written into ``path``, a .npy file [nRows][ncol][nChains] opened with
         numpy.lib.format.open_memmap, by a retire thread (which waits for the copy and deals the rows to
-        the writer threads).  The pinned ring is PIN_SLOTS (two; MCMCN_STORE_PIN_SLOTS) chunks deep: the thread
-        that launches the kernels runs PIN_SLOTS - 1 chunks ahead of the writers and then waits for a slot -- its
-        run-ahead being throttled, the device has the next chunk's launches queued meanwhile.  Device memory is
-        2 x chunkBytes and pinned memory PIN_SLOTS x chunkBytes whatever the run length
+        the writer threads).  The pinned ring mirrors the device ring, one slot per chunk: the thread that
+        launches the kernels runs one chunk ahead of the writers and then waits for a slot -- its run-ahead
+        being throttled, the device has the next chunk's launches queued meanwhile (4 or 6 slots left the
+        sampling loop of config 3 as fast or slower: profiles/experiments/r2_store_pin_slots_ab.log).  Device
+        memory is 2 x chunkBytes and pinned memory the same, whatever the run length
         (posteriorSampling.py:898-909, :933-936 appends a CSV row per retained iteration; this is the
         same stream of rows in binary).  ``Engine.run`` splits its iterations at chunk boundaries;
         ``finish()`` drains the ring.
@@ -164,7 +152,7 @@ class SampleStore(object):
     """
 
     def __init__(self, engine, nRows, dtype=torch.float64, path=None, logLikelihood=False, logLikSink=None,
-                 chunkBytes=128 << 20, parts=1):
+                 chunkBytes=128 << 20):
         self.engine = engine
         self.nRows = int(nRows)
         self.dtype = dtype
@@ -172,7 +160,7 @@ class SampleStore(object):
         self._stopPrefault = False
         self.waitedForWriters = 0.0                 # seconds the launching thread stood waiting for a pinned slot
         self.retireWaitedForDevice = 0.0            # seconds the retire thread waited for chunks to leave the device
-        self.retireWrote = 0.0                      # seconds it spent writing them into the file(s)
+        self.retireWrote = 0.0                      # seconds it spent writing them into the file
         self.path = path
         self.streamed = path is not None
         self.logLikSink = logLikSink
@@ -193,7 +181,6 @@ class SampleStore(object):
             (self.logLik.numel() * 8 if self.logLik is not None else 0)
         if self.streamed:
             self._chunk, self._fill, self._done = 0, 0, 0          # ring position; rows already handed to the sink
-            self.pinSlots = max(2, min(PIN_SLOTS, -(-self.nRows // self.chunkRows)))
             self._side = torch.cuda.Stream(dev)
             # The pinned staging buffers (2 x chunkBytes: 0.6 s of cudaHostAlloc at 1 GB) are allocated by a background
             # thread: the first chunk is full only after the burn-in, so the chains start without waiting for them.
@@ -202,28 +189,20 @@ class SampleStore(object):
             def allocatePinned():
                 torch.cuda.set_device(dev)                          # the thread's own current device (default: 0)
                 pin = [torch.empty((self.chunkRows, engine.nCol, S), dtype=dtype, pin_memory=True)
-                       for _ in range(self.pinSlots)]
+                       for _ in range(2)]
                 pinLL = [torch.empty((self.chunkRows, engine.nObservations, S), dtype=torch.float64, pin_memory=True)
-                         for _ in range(self.pinSlots)] if logLikelihood else None
+                         for _ in range(2)] if logLikelihood else None
                 self._pin, self._pinLL = pin, pinLL
             self._pinThread = threading.Thread(target=allocatePinned, daemon=True)
             self._pinThread.start()
-            self._copied = [None, None]                             # per device chunk: event of its copy to the host
-            self._written = [None] * self.pinSlots                  # per pinned slot: future of the retire job that reads it
-            self._flushes = 0
+            self._copied = [None, None]                             # per chunk: event of its copy to the pinned slot
+            self._written = [None, None]                            # per chunk: future of the retire job reading its slot
             import concurrent.futures
             self._writers = concurrent.futures.ThreadPoolExecutor(max_workers=WRITER_THREADS)
             self._retirer = concurrent.futures.ThreadPoolExecutor(max_workers=1)     # one thread: chunks retire in order
             npdt = numpy.float64 if dtype == torch.float64 else numpy.float32
-            # ``parts`` files, each [nRows][ncol][a contiguous range of the chains]: a tmpfs file's pages are
-            # allocated at 8 GB/s however many threads ask (measured on the GPU box, tools/store_populate_probe.py:
-            # 8.3 GB/s for one file, 16.3 for two, 17.8 for four).  An option for stores whose populating threads
-            # cannot stay ahead of the writers; one file by default (at config 3 it made no difference)
-            parts = int(max(1, min(parts, engine.nChains)))
-            self.partChains = [((engine.nChains * k) // parts, (engine.nChains * (k + 1)) // parts) for k in range(parts)]
-            self.partFiles = [path] if parts == 1 else [path[:-4] + ".part%d.npy" % k for k in range(parts)]
-            self.sinks = [numpy.lib.format.open_memmap(f, mode="w+", dtype=npdt, shape=(self.nRows, engine.nCol, c1 - c0))
-                          for f, (c0, c1) in zip(self.partFiles, self.partChains)]
+            self.sink = numpy.lib.format.open_memmap(path, mode="w+", dtype=npdt,
+                                                     shape=(self.nRows, engine.nCol, engine.nChains))
             self._prefaulters = [threading.Thread(target=self._prefault, args=(k, PREFAULT_THREADS), daemon=True)
                                  for k in range(PREFAULT_THREADS)]
             for t in self._prefaulters:
@@ -238,14 +217,9 @@ class SampleStore(object):
         try:
             libc = ctypes.CDLL(None, use_errno=True)
             page = os.sysconf("SC_PAGE_SIZE")
-            nParts = len(self.sinks)
-            if k >= nParts * (nThreads // nParts) and nThreads >= nParts:
-                return                                              # threads beyond an even share per file
-            sink = self.sinks[k % nParts]                           # this thread's file; its rank among that file's threads
-            k, nThreads = k // nParts, max(1, nThreads // nParts)
-            addr = sink.ctypes.data
+            addr = self.sink.ctypes.data
             lo = addr - addr % page
-            end = addr + sink.nbytes
+            end = addr + self.sink.nbytes
             step = 64 << 20
             lo += k * step
             while lo < end and not self._stopPrefault:
@@ -288,11 +262,9 @@ class SampleStore(object):
             self._pinThread = None
             if self._pin is None:
                 raise RuntimeError("could not allocate the pinned staging buffers of the sample store")
-        slot = self._flushes % self.pinSlots
-        self._flushes += 1
-        if self._written[slot] is not None:         # this pinned slot is still being written to the file: a whole ring behind
+        if self._written[c] is not None:            # its pinned slot is still being written out: a whole ring behind
             t0 = time.perf_counter()
-            self._written[slot].result()            # (re-raises what the retire thread raised)
+            self._written[c].result()               # (re-raises what the retire thread raised)
             self.waitedForWriters += time.perf_counter() - t0
         main = torch.cuda.current_stream(self.engine.device)
         filled = torch.cuda.Event()
@@ -300,13 +272,13 @@ class SampleStore(object):
         self._side.wait_event(filled)
         r0 = c * self.chunkRows
         with torch.cuda.stream(self._side):
-            self._pin[slot][:n].copy_(self.tensor[r0:r0 + n], non_blocking=True)
+            self._pin[c][:n].copy_(self.tensor[r0:r0 + n], non_blocking=True)
             if self.logLik is not None:
-                self._pinLL[slot][:n].copy_(self.logLik[r0:r0 + n], non_blocking=True)
+                self._pinLL[c][:n].copy_(self.logLik[r0:r0 + n], non_blocking=True)
             done = torch.cuda.Event()
             done.record(self._side)
         self._copied[c] = done
-        self._written[slot] = self._retirer.submit(self._retire, (slot, n, self._done, done))
+        self._written[c] = self._retirer.submit(self._retire, (c, n, self._done, done))
         self._done += n
         self._chunk, self._fill = 1 - c, 0
         if self._copied[self._chunk] is not None:    # the chains may overwrite the other chunk once it has left the device
@@ -330,8 +302,7 @@ class SampleStore(object):
 
         def put(job):
             r, k0, k1 = job
-            for sink, (c0, c1) in zip(self.sinks, self.partChains):
-                sink[row0 + r, k0:k1] = src[r, k0:k1, c0:c1]
+            self.sink[row0 + r, k0:k1] = src[r, k0:k1, :nC]
         if len(jobs) > 1:
             list(self._writers.map(put, jobs))
         else:
@@ -355,8 +326,7 @@ class SampleStore(object):
             self._stopPrefault = True
             for t in self._prefaulters:
                 t.join()
-            for sink in self.sinks:
-                sink.flush()
+            self.sink.flush()
         elif self.logLik is not None and self.logLikSink is not None:
             n = len(self.iterations)
             if n:
@@ -365,8 +335,7 @@ class SampleStore(object):
     def hostArray(self):
         """[rows][ncol][nChains] numpy array (the file's memmap when streamed, after finish())."""
         if self.streamed:
-            n = len(self.iterations)
-            return self.sinks[0][:n] if len(self.sinks) == 1 else numpy.concatenate([sk[:n] for sk in self.sinks], axis=2)
+            return self.sink[:len(self.iterations)]
         return self.tensor[:len(self.iterations), :, :self.engine.nChains].cpu().numpy()
 
 

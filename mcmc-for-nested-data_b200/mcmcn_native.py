@@ -4,6 +4,9 @@ Thin by design (north star (5)): structs mirror the header one to one, every cal
 checks the return code and raises with mcmcn_last_error().  There is no CPU
 fallback: if the library is missing or fails to load, importing callers get a
 RuntimeError telling them to run ``python __graft_entry__.py``.
+
+It also holds the host helpers that engine, posteriorSampling and sampleDiagnosis share: tensor
+pointers for the ABI, the rank / world query, the contiguous chain-range rule and the host-thread count.
 """
 
 import ctypes
@@ -167,3 +170,29 @@ def check(rc):
 
 def call(name, *args):
     check(getattr(load(), name)(*args))
+
+
+# ---- host helpers shared by engine, posteriorSampling and sampleDiagnosis
+def _ptr(t):
+    """Device pointer of a tensor for the C ABI (None passes NULL)."""
+    return ctypes.c_void_p(t.data_ptr()) if t is not None else None
+
+
+def _rankWorld():
+    """(rank, world size) under torch.distributed, (0, 1) without it."""
+    import torch.distributed as dist
+    if dist.is_available() and dist.is_initialized():
+        return dist.get_rank(), dist.get_world_size()
+    return 0, 1
+
+
+def chainRange(n, rank, world):
+    """Contiguous slice [lo, hi) of n items (chains; keys in the diagnostics' key-partitioned exchange) that a
+    rank owns."""
+    return (n * rank) // world, (n * (rank + 1)) // world
+
+
+def _hostThreads(env):
+    """Host copy threads of this process: an even share of the cores among the ranks of this box, 2..8."""
+    share = (os.cpu_count() or 4) // max(1, int(os.environ.get("LOCAL_WORLD_SIZE", "1")))
+    return int(os.environ.get(env, max(2, min(8, share // 2))))

@@ -28,6 +28,7 @@ import numpy
 import torch
 
 from engine import Engine, SampleStore, burnThin, retainedIterations
+from mcmcn_native import _rankWorld, chainRange
 from objectives import Objective
 
 # above this many retained values (rows x columns x chains) the samples go to the binary store
@@ -37,8 +38,6 @@ LOGLIK_VALUE_LIMIT = int(os.environ.get("MCMCN_LOGLIK_LIMIT", 200000000))
 # the binary store keeps the chains' FP64 values; "float32" (6e-8 relative, below the reference's "%f"
 # for |values| < 16) is an explicit opt-in that the manifest records
 STORE_DTYPE = os.environ.get("MCMCN_STORE_DTYPE", "float64")
-# files a single process writes its binary store as, by chain range (samples.part<k>.npy when more than one)
-STORE_PARTS = 1
 
 
 def samplePosterior(nChains, nIter, nSamples,
@@ -114,7 +113,7 @@ def _sampleShard(rank, world, nChains, nIter, burn, thin, parameterName, nGroups
                  startingPointValueRange, displayProgress, loggingLevel, logger):
     """This rank's chains (contiguous global ids; Philox and the start-state streams are keyed by them):
     start state, Sampler._loop (:862-896), sample files."""
-    lo, hi = (nChains * rank) // world, (nChains * (rank + 1)) // world
+    lo, hi = chainRange(nChains, rank, world)
     myChains = hi - lo
     show = displayProgress and rank == 0
     phases, mark = {}, [time.perf_counter()]
@@ -158,14 +157,9 @@ def _sampleShard(rank, world, nChains, nIter, burn, thin, parameterName, nGroups
     if not useCsv and STORE_DTYPE == "float32":
         storeDtype = torch.float32
     shardFile = "samples.npy" if world == 1 else "samples.rank%d.npy" % rank
-    # MCMCN_STORE_PARTS=k: a single process writes its store as k files by chain range (engine.SampleStore: a tmpfs
-    # file's pages are allocated at a fixed rate per file).  Off by default: at config 3 the writers are not what
-    # the sampling loop waits for (retire thread: 1.2 s writing, 1.7 s waiting for the device), measured both ways.
-    parts = int(os.environ.get("MCMCN_STORE_PARTS", STORE_PARTS))
     store = SampleStore(eng, max(len(retained), 1), storeDtype,
                         path=None if useCsv else os.path.join(sampleDirectory, shardFile),
-                        logLikelihood=bool(saveLogLikelihood), logLikSink=appendLogLikelihood,
-                        parts=parts if world == 1 else 1)
+                        logLikelihood=bool(saveLogLikelihood), logLikSink=appendLogLikelihood)
 
     # ---- Sampler._loop (:862-896): one call per progress mark; the store splits it where a chunk is full
     stops = set([nIter])
@@ -209,14 +203,12 @@ def _sampleShard(rank, world, nChains, nIter, burn, thin, parameterName, nGroups
     global lastRun
     lastRun = {"engine": eng, "store": store, "retained": retained, "chains": (lo, hi),
                "sampling_seconds": elapsed.total_seconds(), "store_device_bytes": store.deviceBytes,
-               "store_pinned_bytes": (store.deviceBytes // 2) * store.pinSlots if store.streamed else 0,
+               "store_pinned_bytes": store.deviceBytes if store.streamed else 0,    # two chunks, as on the device
                "phases": phases}
     _barrier(world)                                                 # every shard file is complete
     if not useCsv and rank == 0:
-        parted = [{"file": os.path.basename(f), "chains": [int(c0), int(c1)]}
-                  for f, (c0, c1) in zip(store.partFiles, store.partChains)] if world == 1 else None
         writeManifest(sampleDirectory, header, retained, nChains, world, pooling,
-                      "float64" if storeDtype == torch.float64 else "float32", shards=parted)
+                      "float64" if storeDtype == torch.float64 else "float32")
     phase("files")
     return elapsed
 
@@ -248,15 +240,11 @@ def writeSampleCsv(path, chain, header, iterations, rows):
             h.write("\n")
 
 
-def writeManifest(sampleDirectory, header, iterations, nChains, world, pooling, dtype, shards=None):
+def writeManifest(sampleDirectory, header, iterations, nChains, world, pooling, dtype):
     """``sample/manifest.json``: what sampleDiagnosis.openSamples reads.  One shard file per rank, each
-    [rows][columns][chains of that rank] (.npy), chains split contiguously over the ranks; a single process
-    names its own file(s) (``shards``: one, or two by chain range for a large store)."""
-    if shards is None:
-        shards = []
-        for r in range(world):
-            lo, hi = (nChains * r) // world, (nChains * (r + 1)) // world
-            shards.append({"file": "samples.npy" if world == 1 else "samples.rank%d.npy" % r, "chains": [lo, hi]})
+    [rows][columns][chains of that rank] (.npy), chains split contiguously over the ranks (chainRange)."""
+    shards = [{"file": "samples.npy" if world == 1 else "samples.rank%d.npy" % r,
+               "chains": list(chainRange(nChains, r, world))} for r in range(world)]
     man = {"format": "mcmcn-samples-2", "header": list(header), "iterations": list(map(int, iterations)),
            "nChains": int(nChains), "pooling": pooling, "dtype": dtype,
            "layout": "[rows][columns][chains]", "shards": shards}
@@ -267,13 +255,6 @@ def writeManifest(sampleDirectory, header, iterations, nChains, world, pooling, 
 
 
 # ------------------------------------------------------------------------------ plumbing
-def _rankWorld():
-    import torch.distributed as dist
-    if dist.is_available() and dist.is_initialized():
-        return dist.get_rank(), dist.get_world_size()
-    return 0, 1
-
-
 def _barrier(world):
     if world > 1:
         import torch.distributed as dist

@@ -24,10 +24,7 @@ import pandas
 import torch
 
 import mcmcn_native as nat
-
-
-def _ptr(t):
-    return ctypes.c_void_p(t.data_ptr()) if t is not None else None
+from mcmcn_native import _hostThreads, _ptr, _rankWorld, chainRange
 
 
 def _device():
@@ -58,32 +55,33 @@ def _sortedMedianHdi(x, hdi_p):
     return _sortedMedianHdiDevice(x, hdi_p).cpu().numpy()
 
 
-def keyRange(nKeys, rank, world):
-    """Contiguous slice [lo, hi) of the keys a rank owns in the key-partitioned exchange."""
-    return (nKeys * rank) // world, (nKeys * (rank + 1)) // world
+def _rankLengths(length, group, device):
+    """Every rank's ``length`` (an int), in rank order: one all-gather."""
+    import torch.distributed as dist
+    lens = [torch.zeros(1, dtype=torch.int64, device=device) for _ in range(dist.get_world_size(group))]
+    dist.all_gather(lens, torch.tensor([length], dtype=torch.int64, device=device), group=group)
+    return [int(v) for v in lens]
 
 
 def exchangeByKey(local, group):
     """Key-partitioned exchange for the pooled order statistics (SURVEY.md section 8e / 8f-3):
     ``local`` is this rank's [n_keys][len_r] draws (len_r may differ between ranks); rank r becomes the
-    owner of keys keyRange(r) and receives every rank's draws of those keys, concatenated in rank
+    owner of keys chainRange(n_keys, r) and receives every rank's draws of those keys, concatenated in rank
     (= chain) order: returns [keys_owned][sum of len_r].  One all-to-all over NVLink with NCCL; backends
     without all-to-all (gloo, used by the CPU tests) run the same exchange as one gather per owner."""
     import torch.distributed as dist
     world, rank = dist.get_world_size(group), dist.get_rank(group)
     nKeys, length = local.shape
-    lens = [torch.zeros(1, dtype=torch.int64, device=local.device) for _ in range(world)]
-    dist.all_gather(lens, torch.tensor([length], dtype=torch.int64, device=local.device), group=group)
-    lens = [int(v) for v in lens]
-    send = [local[slice(*keyRange(nKeys, r, world))].contiguous() for r in range(world)]
-    lo, hi = keyRange(nKeys, rank, world)
+    lens = _rankLengths(length, group, local.device)
+    send = [local[slice(*chainRange(nKeys, r, world))].contiguous() for r in range(world)]
+    lo, hi = chainRange(nKeys, rank, world)
     recv = [torch.empty((hi - lo, lens[r]), dtype=local.dtype, device=local.device) for r in range(world)]
     if dist.get_backend(group) == "nccl":
         dist.all_to_all(recv, send, group=group)
     else:
         most = max(lens)                                 # gather wants equal shapes: pad to the longest, trim after
         for r in range(world):
-            klo, khi = keyRange(nKeys, r, world)
+            klo, khi = chainRange(nKeys, r, world)
             padded = torch.zeros((khi - klo, most), dtype=local.dtype, device=local.device)
             padded[:, :length] = send[r]
             got = [torch.empty_like(padded) for _ in range(world)] if r == rank else None
@@ -105,14 +103,13 @@ def pooledMedianHdi(local, hdi_p, group, keySlab=2048):
     for k0 in range(0, nKeys, keySlab):
         k1 = min(nKeys, k0 + keySlab)
         mine = _sortedMedianHdiDevice(exchangeByKey(local[k0:k1], group), hdi_p)     # [keys owned in this slab][3]
-        most = max(keyRange(k1 - k0, r, world)[1] - keyRange(k1 - k0, r, world)[0] for r in range(world))
-        pad = torch.zeros((most, 3), dtype=torch.float64, device=local.device)
+        owned = [chainRange(k1 - k0, r, world) for r in range(world)]
+        pad = torch.zeros((max(hi - lo for lo, hi in owned), 3), dtype=torch.float64, device=local.device)
         pad[:mine.shape[0]] = mine
         parts = [torch.empty_like(pad) for _ in range(world)]
         dist.all_gather(parts, pad, group=group)
-        for r in range(world):
-            lo, hi = keyRange(k1 - k0, r, world)
-            out[k0 + lo:k0 + hi] = parts[r][:hi - lo]
+        for (lo, hi), part in zip(owned, parts):
+            out[k0 + lo:k0 + hi] = part[:hi - lo]
     return out
 
 
@@ -126,20 +123,7 @@ def computeHpdInterval(samples, hdi_p=95):
 
 # ------------------------------------------------------------------------------ where the draws come from
 SLAB_BYTES = int(os.environ.get("MCMCN_DIAG_SLAB_BYTES", 1 << 30))     # device bytes of half-chains per slab of keys
-def _hostThreads(env):
-    """Host copy threads of this process: an even share of the cores among the ranks of this box, 2..8."""
-    share = (os.cpu_count() or 4) // max(1, int(os.environ.get("LOCAL_WORLD_SIZE", "1")))
-    return int(os.environ.get(env, max(2, min(8, share // 2))))
-
-
 STAGE_THREADS = _hostThreads("MCMCN_DIAG_THREADS")
-
-
-def _rankWorld():
-    import torch.distributed as dist
-    if dist.is_available() and dist.is_initialized():
-        return dist.get_rank(), dist.get_world_size()
-    return 0, 1
 
 
 class SampleSource(object):
@@ -155,7 +139,7 @@ class SampleSource(object):
         self.nRows = int(nRows)
         self.chains = [c for _, ids in blocks for c in ids]
         self.nChains = len(self.chains)
-        self._pins, self._pool, self._stageKeys = {}, None, 1
+        self._pins, self._pool = {}, None
 
     @classmethod
     def fromArray(cls, samples, keys, chains=None):
@@ -165,11 +149,17 @@ class SampleSource(object):
         block = numpy.ascontiguousarray(numpy.transpose(samples, (1, 2, 0)))       # [rows][keys][chains]
         return cls(keys, [(block, list(chains) if chains is not None else list(range(nC)))], rows)
 
+    @classmethod
+    def fromStore(cls, storeTensor, nRows, nChains):
+        """The device-resident sample store [rows][ncol][S] (engine.SampleStore.tensor), its first nChains chains."""
+        return cls(["c%d" % k for k in range(storeTensor.shape[1])], [(storeTensor, list(range(nChains)))], nRows)
+
     def stage(self, k0, k1, slot=0):
         """Host half of halfChains: the columns k0..k1 of every host block (numpy array or memmap of a shard
         file) copied into pinned memory, rows split over a few threads (numpy copies release the GIL; one
         thread gathers about 4 GB/s out of a memory-mapped file).  Two slots, so that the next slab can be
-        staged while the device works on this one.  Returns one pinned tensor (or None: device block) per block."""
+        staged while the device works on this one; a slot's buffer is kept while it is large enough (the slabs
+        of a pass are all of one size but the last).  Returns one pinned tensor (or None: device block) per block."""
         n = self.nRows // 2
         out = []
         for bi, (arr, ids) in enumerate(self.blocks):
@@ -181,7 +171,7 @@ class SampleSource(object):
             key = (bi, slot)
             pin = self._pins.get(key)
             if pin is None or pin.dtype != tdt or pin.numel() < 2 * n * nk * nC:
-                pin = torch.empty((2 * n * max(nk, self._stageKeys) * nC,), dtype=tdt)
+                pin = torch.empty((2 * n * nk * nC,), dtype=tdt)
                 if torch.cuda.is_available():
                     pin = pin.pin_memory()
                 self._pins[key] = pin
@@ -300,15 +290,12 @@ def gatherShards(t, group):
     """all-gather a [n_keys][m_local][..] tensor along the half-chain axis (dim 1), rank order; ranks may
     hold different numbers of chains (padded to the largest for the collective, trimmed after)."""
     import torch.distributed as dist
-    world = dist.get_world_size(group)
-    sizes = [torch.zeros(1, dtype=torch.int64, device=t.device) for _ in range(world)]
-    dist.all_gather(sizes, torch.tensor([t.shape[1]], dtype=torch.int64, device=t.device), group=group)
-    sizes = [int(v) for v in sizes]
+    sizes = _rankLengths(t.shape[1], group, t.device)
     most = max(sizes)
     if t.shape[1] < most:
         pad = torch.zeros((t.shape[0], most - t.shape[1]) + tuple(t.shape[2:]), dtype=t.dtype, device=t.device)
         t = torch.cat([t, pad], dim=1)
-    parts = [torch.empty_like(t) for _ in range(world)]
+    parts = [torch.empty_like(t) for _ in sizes]
     dist.all_gather(parts, t.contiguous(), group=group)
     return torch.cat([p[:, :sz] for p, sz in zip(parts, sizes)], dim=1).contiguous()
 
@@ -332,8 +319,9 @@ def _slabKeys(nKeys, mLocal, n):
     return int(max(1, min(nKeys, SLAB_BYTES // (8 * per), ((1 << 31) - 1) // per, 65535)))
 
 
-def _convergenceSlab(x, group):
-    """R-hat quadruple [nk][4], per-lag sums and ESS of one slab of half-chains x [nk][mLocal][n]."""
+def _convergenceSlab(x, group, rh):
+    """R-hat quadruple of one slab of half-chains x [nk][mLocal][n], written into rh [nk][4]; returns the
+    per-lag sums [nk][n] (over all ranks' chains under ``group``) and the number of half-chains m."""
     dev = x.device
     nk, mL, n = x.shape
     st = _stream(dev)
@@ -346,9 +334,68 @@ def _convergenceSlab(x, group):
     if group is not None:
         mean, var, vario = mergeShards(mean, var, vario, group)
     m = mean.shape[1]
-    rh = torch.empty((nk, 4), dtype=f64, device=dev)
     nat.call("mcmcn_diag_rhat", _ptr(mean), _ptr(var), nk, m, n, _ptr(rh), st)
-    return rh, vario, m
+    return vario, m
+
+
+def _slabStatistics(source, dev, group, convergence=False, orderStatistics=False, rho=None, hdi_p=95, timing=None):
+    """One pass of the diagnostics over a SampleSource, a slab of keys at a time (_slabKeys); while the device works
+    on a slab, a host thread stages the next slab's host rows (sources with host blocks only).  ``convergence``:
+    the R-hat quadruple (B, W, vhat, R-hat) and the ESS of every key, and its autocorrelations copied into
+    ``rho`` (host [keys][n]) if given; ``orderStatistics``: the median and HDI of every key's pooled draws.
+    Under ``group`` (chains sharded over the ranks) ``timing`` receives what this rank exchanged.  Returns device
+    (rhat [keys][4], ess [keys], medianHdi [keys][3]), None for what was not asked."""
+    import concurrent.futures
+    st = _stream(dev)
+    f64 = torch.float64
+    nKeys, mL, n = len(source.keys), 2 * source.nChains, source.nRows // 2
+    rh = torch.empty((nKeys, 4), dtype=f64, device=dev) if convergence else None
+    ess = torch.empty((nKeys,), dtype=f64, device=dev) if convergence else None
+    mh = torch.empty((nKeys, 3), dtype=f64, device=dev) if orderStatistics else None
+    world = 1
+    if group is not None:
+        import torch.distributed as dist
+        world = dist.get_world_size(group)
+    step = _slabKeys(nKeys, mL, n)
+    slabs = [(k0, min(nKeys, k0 + step)) for k0 in range(0, nKeys, step)]
+    ahead = concurrent.futures.ThreadPoolExecutor(max_workers=1) \
+        if any(not isinstance(arr, torch.Tensor) for arr, _ in source.blocks) else None
+
+    def stage(i):                                                      # slab i's host rows into pinned slot i & 1
+        return ahead.submit(source.stage, *slabs[i], i & 1) if ahead is not None and i < len(slabs) else None
+    pending = stage(0)
+    gathered = exchanged = 0
+    for i, (k0, k1) in enumerate(slabs):
+        nk = k1 - k0
+        staged = pending.result() if pending is not None else None
+        pending = stage(i + 1)                                         # the next slab's rows leave the files meanwhile
+        x = source.halfChains(k0, k1, dev, staged)                     # [nk][mL][n]
+        r = None
+        if convergence:
+            vario, m = _convergenceSlab(x, group, rh[k0:k1])
+            r = torch.empty((nk, n), dtype=f64, device=dev) if rho is not None else None
+            nat.call("mcmcn_diag_ess", _ptr(vario), _ptr(rh[k0:k1]), nk, m, n, _ptr(r), _ptr(ess[k0:k1]), st)
+            if group is not None:       # what mergeShards received: all m half-chains' means + variances, every rank's per-lag sums
+                gathered += nk * (2 * m + n * world) * 8
+        if orderStatistics:
+            pooled = x.reshape(nk, mL * n)                             # sorted in place: x is not needed again
+            if group is not None:       # key-partitioned all-to-all: no rank holds every key's pooled draws
+                mh[k0:k1] = pooledMedianHdi(pooled, hdi_p, group)
+                exchanged += pooled.numel() * 8 * (world - 1) // world     # what this rank sent to the other owners
+            else:
+                mh[k0:k1] = _sortedMedianHdiDevice(pooled, hdi_p)
+            del pooled
+        if r is not None:
+            rho[k0:k1] = r.cpu().numpy()
+        del x
+    if ahead is not None:
+        ahead.shutdown()
+    if timing is not None:
+        if convergence:
+            timing["gathered_bytes"], timing["slabs"] = gathered, len(slabs)
+        if orderStatistics:
+            timing["exchanged_bytes"] = exchanged
+    return rh, ess, mh
 
 
 def convergenceFromStore(storeTensor, nRows, nChains, group=None, timing=None):
@@ -359,30 +406,11 @@ def convergenceFromStore(storeTensor, nRows, nChains, group=None, timing=None):
     ``group`` every rank holds a shard of the chains and the half-chain moments and per-lag sums
     are exchanged by one NCCL all-gather per slab (mergeShards); ``timing`` (a dict) then
     receives the bytes this rank gathered.  Returns (rhat[ncol], ess[ncol]) as device tensors."""
-    n = int(nRows) // 2
-    if n < 2:
+    if int(nRows) // 2 < 2:
         raise ValueError("need at least 4 retained rows per chain")
-    ncol = storeTensor.shape[1]
-    dev = storeTensor.device
-    src = SampleSource(["c%d" % k for k in range(ncol)], [(storeTensor, list(range(nChains)))], 2 * n)
-    rhat = torch.empty((ncol,), dtype=torch.float64, device=dev)
-    ess = torch.empty((ncol,), dtype=torch.float64, device=dev)
-    step = _slabKeys(ncol, 2 * nChains, n)
-    gathered = 0
-    for k0 in range(0, ncol, step):
-        k1 = min(ncol, k0 + step)
-        x = src.halfChains(k0, k1, dev)
-        rh, vario, m = _convergenceSlab(x, group)
-        nat.call("mcmcn_diag_ess", _ptr(vario), _ptr(rh), k1 - k0, m, n, None, _ptr(ess[k0:k1]), _stream(dev))
-        rhat[k0:k1] = rh[:, 3]
-        if group is not None:                      # what mergeShards received: means + variances of all m half-chains, per-lag sums of every rank
-            import torch.distributed as dist
-            gathered += (k1 - k0) * (2 * m + n * dist.get_world_size(group)) * 8
-        del x
-    if timing is not None:
-        timing["gathered_bytes"] = gathered
-        timing["slabs"] = (ncol + step - 1) // step
-    return rhat, ess
+    rh, ess, _ = _slabStatistics(SampleSource.fromStore(storeTensor, nRows, nChains), storeTensor.device, group,
+                                 convergence=True, timing=timing)
+    return rh[:, 3].contiguous(), ess
 
 
 def orderStatisticsFromStore(storeTensor, nRows, nChains, hdi_p=95, group=None, timing=None):
@@ -390,32 +418,24 @@ def orderStatisticsFromStore(storeTensor, nRows, nChains, hdi_p=95, group=None, 
     store, pooled over all chains and rows, in slabs of columns.  With ``group`` the pooled draws of a
     slab go through the key-partitioned all-to-all (pooledMedianHdi): no rank ever holds all draws of all
     columns.  Returns device [ncol][3] = median, HDI lower, HDI upper."""
-    n = int(nRows) // 2
-    ncol = storeTensor.shape[1]
-    dev = storeTensor.device
-    src = SampleSource(["c%d" % k for k in range(ncol)], [(storeTensor, list(range(nChains)))], 2 * n)
-    out = torch.empty((ncol, 3), dtype=torch.float64, device=dev)
-    step = _slabKeys(ncol, 2 * nChains, n)
-    exchanged = 0
-    for k0 in range(0, ncol, step):
-        k1 = min(ncol, k0 + step)
-        pooled = src.halfChains(k0, k1, dev).reshape(k1 - k0, 2 * nChains * n)
-        if group is not None:
-            import torch.distributed as dist
-            world = dist.get_world_size(group)
-            out[k0:k1] = pooledMedianHdi(pooled, hdi_p, group)
-            exchanged += pooled.numel() * 8 * (world - 1) // world          # what this rank sent to the other owners
+    return _slabStatistics(SampleSource.fromStore(storeTensor, nRows, nChains), storeTensor.device, group,
+                           orderStatistics=True, hdi_p=hdi_p, timing=timing)[2]
+
+
+def _resolveSource(sampleDirectory, samples, keys, group, source):
+    """(SampleSource, process group) of Diagnostic's / Summary's arguments: ``source`` as given, ``samples`` in
+    memory, or what openSamples finds under ``sampleDirectory`` -- under torch.distributed with one shard per
+    rank each rank opens its own, and the ranks exchange over the world group unless ``group`` is given."""
+    if source is None:
+        if samples is not None:
+            source = SampleSource.fromArray(samples, keys)
         else:
-            out[k0:k1] = _sortedMedianHdiDevice(pooled, hdi_p)
-        del pooled
-    if timing is not None:
-        timing["exchanged_bytes"] = exchanged
-    return out
-
-
-def chainRange(nChains, rank, world):
-    """Contiguous global chain ids [lo, hi) of a rank."""
-    return (nChains * rank) // world, (nChains * (rank + 1)) // world
+            rank, world = _rankWorld()
+            source = openSamples(sampleDirectory, rank, world)
+            if source.sharded and group is None:
+                import torch.distributed as dist
+                group = dist.group.WORLD
+    return source, group
 
 
 class Diagnostic(object):
@@ -424,18 +444,8 @@ class Diagnostic(object):
         ``samples`` = array [nChains][rows][nKeys] (+ ``keys``) already in memory, or a SampleSource.
         ``group``: a torch.distributed process group whose ranks each hold a shard of the
         chains; results are then over all ranks' chains."""
-        if source is None:
-            if samples is not None:
-                source = SampleSource.fromArray(samples, keys)
-            else:
-                rank, world = _rankWorld()
-                source = openSamples(sampleDirectory, rank, world)
-                if source.sharded and group is None:
-                    import torch.distributed as dist
-                    group = dist.group.WORLD
-        self._source = source
-        self._keys = list(source.keys)
-        self._group = group
+        self._source, self._group = _resolveSource(sampleDirectory, samples, keys, group, source)
+        self._keys = list(self._source.keys)
         self._organiseSamples()
         self._done = False
         self._hdiP = 95
@@ -464,46 +474,17 @@ class Diagnostic(object):
     def _compute(self):
         if self._done:
             return
-        dev = _device()
-        nKeys, mL, n = len(self._keys), self._mLocal, self._n
-        st = _stream(dev)
-        f64 = torch.float64
-        rh_h = numpy.empty((nKeys, 4))
-        ess_h = numpy.empty(nKeys)
-        mh = numpy.empty((nKeys, 3))
-        self._rhoArr = numpy.empty((nKeys, n))
-        step = _slabKeys(nKeys, mL, n)
-        self._source._stageKeys = step
-        import concurrent.futures
-        ahead = concurrent.futures.ThreadPoolExecutor(max_workers=1)
-        slabs = [(k0, min(nKeys, k0 + step)) for k0 in range(0, nKeys, step)]
-        pending = ahead.submit(self._source.stage, slabs[0][0], slabs[0][1], 0)
-        for i, (k0, k1) in enumerate(slabs):
-            nk = k1 - k0
-            staged = pending.result()
-            if i + 1 < len(slabs):                                     # the next slab's rows leave the files meanwhile
-                pending = ahead.submit(self._source.stage, slabs[i + 1][0], slabs[i + 1][1], (i + 1) & 1)
-            x = self._source.halfChains(k0, k1, dev, staged)           # [nk][mL][n]
-            rh, vario, m = _convergenceSlab(x, self._group)
-            ess = torch.empty((nk,), dtype=f64, device=dev)
-            rho = torch.empty((nk, n), dtype=f64, device=dev)
-            nat.call("mcmcn_diag_ess", _ptr(vario), _ptr(rh), nk, m, n, _ptr(rho), _ptr(ess), st)
-            pooled = x.reshape(nk, mL * n)                             # sorted in place: x is not needed again
-            if self._group is not None:   # key-partitioned all-to-all: no rank holds every key's pooled draws
-                mh[k0:k1] = pooledMedianHdi(pooled, self._hdiP, self._group).cpu().numpy()
-            else:
-                mh[k0:k1] = _sortedMedianHdi(pooled, self._hdiP)
-            rh_h[k0:k1], ess_h[k0:k1] = rh.cpu().numpy(), ess.cpu().numpy()
-            self._rhoArr[k0:k1] = rho.cpu().numpy()
-            del x, pooled
-        ahead.shutdown()
+        self._rhoArr = numpy.empty((len(self._keys), self._n))
+        stats = _slabStatistics(self._source, _device(), self._group, convergence=True, orderStatistics=True,
+                                rho=self._rhoArr, hdi_p=self._hdiP)
+        rh, ess, mh = (t.cpu().numpy() for t in stats)
         k = self._keys
-        self._B = dict(zip(k, rh_h[:, 0]))
-        self._W = dict(zip(k, rh_h[:, 1]))
-        self._vhat = dict(zip(k, rh_h[:, 2]))
-        self._rhat = dict(zip(k, rh_h[:, 3]))
+        self._B = dict(zip(k, rh[:, 0]))
+        self._W = dict(zip(k, rh[:, 1]))
+        self._vhat = dict(zip(k, rh[:, 2]))
+        self._rhat = dict(zip(k, rh[:, 3]))
         self._rho = dict(zip(k, self._rhoArr))
-        self._effectiveN = dict(zip(k, ess_h))
+        self._effectiveN = dict(zip(k, ess))
         self._median = dict(zip(k, mh[:, 0]))
         self._hdi = dict((key, (mh[i, 1], mh[i, 2])) for i, key in enumerate(k))
         self._done = True
@@ -633,15 +614,7 @@ class Summary(object):
     second step runs on the full vector: the result equals the single-process one bit for bit."""
 
     def __init__(self, sampleDirectory=None, samples=None, keys=None, group=None, source=None):
-        if source is None:
-            if samples is not None:
-                source = SampleSource.fromArray(samples, keys)
-            else:
-                rank, world = _rankWorld()
-                source = openSamples(sampleDirectory, rank, world)
-                if source.sharded and group is None:
-                    import torch.distributed as dist
-                    group = dist.group.WORLD
+        source, group = _resolveSource(sampleDirectory, samples, keys, group, source)
         keys = source.keys
         self._n = source.nRows
         names = sorted(set(name.split("[")[0] for name in keys if "[" in name))

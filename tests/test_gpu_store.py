@@ -3,7 +3,6 @@ binary store, the manifest with its shards, and the diagnostics reading it in sl
 resident store / in-memory path on the same Philox streams."""
 
 import json
-import os
 
 import numpy
 import pytest
@@ -58,37 +57,30 @@ def test_streamed_store_equals_resident_store(dtype, tmp_path):
     assert got["streamed"][1].shape == (nRows, 120, 37) and numpy.isfinite(got["streamed"][1]).all()
 
 
-def test_store_in_two_files_by_chain_range_equals_one_file(tmp_path, monkeypatch):
-    """A single-process store written as two files by chain range (an option: a tmpfs file's pages are allocated at
-    a fixed rate per file): the same rows land in samples.part0/1.npy, the manifest names both with their chain
-    ranges, and loadSamples / Diagnostic over the two files equal those over the one file."""
+def test_diagnostic_over_several_shard_files_equals_one_array(tmp_path, monkeypatch):
+    """One process diagnosing a store of several shard files (a multi-rank run's store, read afterwards): the
+    half-chains of every slab are gathered from all the shards, and R-hat, ESS, median and HDI equal those over
+    the same draws as one array in memory.  Slabs of 4 of the 6 keys, so that a pinned slot is reused by a
+    smaller slab."""
     import posteriorSampling as ps
     import sampleDiagnosis as sd
-    from objectives import Objective
-    obj, names, nResp, ranges = parity.syntheticRegression(G=5, R=12, K=2)
-    handle = Objective.linear_regression(obj.X, obj.y)
-    args = (7, 300, 60, names, 5, nResp, "partial", handle)
-    kw = dict(saveLogLikelihood=False, startingPointValueRange=ranges, displayProgress=False)
-    monkeypatch.setattr(ps, "CSV_VALUE_LIMIT", 0)
-    ps.samplePosterior(*args, str(tmp_path / "one"), **kw)
-    assert os.path.exists(str(tmp_path / "one/sample/samples.npy"))
-    monkeypatch.setattr(ps, "STORE_PARTS", 2)
-    ps.samplePosterior(*args, str(tmp_path / "two"), **kw)
-    man = json.load(open(str(tmp_path / "two/sample/manifest.json")))
-    assert man["shards"] == [{"file": "samples.part0.npy", "chains": [0, 3]}, {"file": "samples.part1.npy", "chains": [3, 7]}]
-    assert not os.path.exists(str(tmp_path / "two/sample/samples.npy"))
-    whole = numpy.load(str(tmp_path / "one/sample/samples.npy"))
-    numpy.testing.assert_array_equal(numpy.load(str(tmp_path / "two/sample/samples.part0.npy")), whole[:, :, :3])
-    numpy.testing.assert_array_equal(numpy.load(str(tmp_path / "two/sample/samples.part1.npy")), whole[:, :, 3:])
-    numpy.testing.assert_array_equal(ps.lastRun["store"].hostArray(), whole)
-    k1, a1, c1 = sd.loadSamples(str(tmp_path / "one/sample/"))
-    k2, a2, c2 = sd.loadSamples(str(tmp_path / "two/sample/"))
-    assert k1 == k2 and c1 == c2 == list(range(7))
-    numpy.testing.assert_array_equal(a1, a2)
-    d1, d2 = sd.Diagnostic(str(tmp_path / "one/sample/")), sd.Diagnostic(str(tmp_path / "two/sample/"))
-    for k in k1:
-        assert d1.rhat[k] == d2.rhat[k] and d1.effectiveN[k] == d2.effectiveN[k]
-        assert d1.median[k] == d2.median[k] and d1.hdi[k] == d2.hdi[k]
+    rs = numpy.random.RandomState(7)
+    rows, nChains, world = 40, 7, 3
+    header = ["a_mu", "a_sigma2", "a[000]", "a[001]", "b[000]", "b[001]"]
+    full = rs.normal(size=(rows, len(header), nChains)).cumsum(axis=0)       # random walks: R-hat well above 1
+    d = str(tmp_path) + "/"
+    for r in range(world):
+        lo, hi = sd.chainRange(nChains, r, world)
+        numpy.save(d + "samples.rank%d.npy" % r, full[:, :, lo:hi])
+    ps.writeManifest(d, header, list(range(rows)), nChains, world, "partial", "float64")
+    monkeypatch.setattr(sd, "SLAB_BYTES", 4 * (2 * nChains) * (rows // 2) * 8)
+    dShards = sd.Diagnostic(d)
+    assert len(dShards._source.blocks) == world
+    monkeypatch.setattr(sd, "SLAB_BYTES", 1 << 30)
+    dOne = sd.Diagnostic(samples=numpy.transpose(full, (2, 0, 1)), keys=header)
+    for k in header:
+        assert dShards.rhat[k] == dOne.rhat[k] and dShards.effectiveN[k] == dOne.effectiveN[k]
+        assert dShards.median[k] == dOne.median[k] and dShards.hdi[k] == dOne.hdi[k]
 
 
 def test_samplePosterior_binary_store_manifest_and_slabbed_diagnostics(tmp_path, monkeypatch, capsys):

@@ -397,10 +397,10 @@ def test_shard_merge_over_gloo_world_size_2(tmp_path):
     numpy.testing.assert_array_equal(a[:70], mean.ravel())
     numpy.testing.assert_array_equal(a[70:140], var.ravel())
     numpy.testing.assert_allclose(a[140:], vario.ravel(), rtol=1e-13)
-    # exchangeByKey: rank r owns keys keyRange(5, r, 2) and holds ALL chains' draws of them, chain order
+    # exchangeByKey: rank r owns keys chainRange(5, r, 2) and holds ALL chains' draws of them, chain order
     import sampleDiagnosis as sd
     for r in range(2):
-        lo, hi = sd.keyRange(5, r, 2)
+        lo, hi = sd.chainRange(5, r, 2)
         numpy.testing.assert_array_equal(numpy.load(tmp_path / ("owned.%d.npy" % r)), x[lo:hi].reshape(hi - lo, -1))
         numpy.testing.assert_array_equal(numpy.load(tmp_path / ("chains.%d.npy" % r)), x[0, 0::2, :])
 
