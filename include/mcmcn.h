@@ -134,7 +134,9 @@ typedef struct mcmcn_model {
      * pooling field is ignored); each sweep then evaluates the proposal's log-likelihood over those
      * groups in parallel (observations x chains across the whole GPU), sums the partial sums in group
      * order per chain and takes the decision in a per-chain kernel (CompletePooling,
-     * posteriorSampling.py:662-685).  `split_scratch`: device, (P + split->n_groups + 3) * stride doubles. */
+     * posteriorSampling.py:662-685); mcmcn_group_loglik evaluates over the same groups.  Environment
+     * variable MCMCN_NO_SPLIT=1 ignores `split` in both.  `split_scratch`: device,
+     * (P + split->n_groups + 3) * stride doubles, working memory of mcmcn_run and mcmcn_group_loglik. */
     const struct mcmcn_model* split;
     double* split_scratch;
 } mcmcn_model;
@@ -216,7 +218,10 @@ int mcmcn_timing_collect(void);
 /* Group log-likelihood of the current state (posteriorSampling.py:629-635 with
  * proposedParameter=None).  out_ll is device [G][S].  If pooled_theta (device
  * [P][S]) is not NULL every group uses those values instead of state.theta
- * (MCMC._mleObjectiveFunction, :1102-1105). */
+ * (MCMC._mleObjectiveFunction, :1102-1105).  With a split model (complete pooling at scale,
+ * mcmcn_model.split) the log-likelihood is evaluated per small group into split_scratch and
+ * out_ll[0][c] is their sum, from 0.0 in group order, for every chain c < n_chains; lanes
+ * from n_chains on are unspecified. */
 int mcmcn_group_loglik(const mcmcn_model* model, const mcmcn_state* state,
                        const double* pooled_theta, double* out_ll, void* stream);
 

@@ -1526,12 +1526,15 @@ __global__ void snapshot_kernel(int P, int G, int partial, int n_chains, int S, 
         if (col0 + k < ncol) store_row[(size_t)(col0 + k) * S + ch] = (TS)v[k];
 }
 
-static __global__ void pooled_nll_kernel(int G, int S, const double* ll, double* out) {
+// out[c] = sum_g ll[g][c] (NEGATE: its negation), from 0.0 in group order: the pooled negative log-likelihood
+// (mcmcn_pooled_nll) and the complete-pooling log-likelihood over the small groups (mcmcn_group_loglik)
+template <bool NEGATE>
+static __global__ void group_sum_kernel(int G, int S, const double* ll, double* out) {
     const int ch = blockIdx.x * blockDim.x + threadIdx.x;
     if (ch >= S) return;
     double s = 0.0;
     for (int g = 0; g < G; ++g) s += ll[(size_t)g * S + ch];
-    out[ch] = -s;
+    out[ch] = NEGATE ? -s : s;
 }
 
 }  // namespace mcmcn

@@ -280,32 +280,49 @@ static int write_retained_row(const KernelSet* ks, const mcmcn_model* m, const m
     return MCMCN_OK;
 }
 
-// Complete pooling with the observations split into small groups (mcmcn_model.split): per sweep
-// propose -> eval over the small groups -> decide.  `mks` is the kernel set of the model m itself
-// (pointwise log-likelihood of the retained rows).
-static int run_complete_split(const KernelSet* mks, const mcmcn_model* m, const mcmcn_state* s, const mcmcn_run_args* r,
-                              cudaStream_t stream) {
+// The split model of complete pooling at scale (mcmcn_model.split), its kernel set and the regions of
+// m->split_scratch: candidate vector [P][S] | log-likelihood per small group [split->n_groups][S] | proposal,
+// uniform and proposal log-prior [3][S].  e is null when m has no split model or MCMCN_NO_SPLIT is set: the
+// single group of all N observations is then evaluated and stepped as it is.
+struct Split {
+    const mcmcn_model* e;
+    const KernelSet* ks;
+    double *cand, *part, *park;
+};
+static int resolve_split(const mcmcn_model* m, const mcmcn_state* s, Split& sp) {
+    memset(&sp, 0, sizeof(sp));
+    if (m->pooling != MCMCN_POOL_COMPLETE || !m->split || getenv("MCMCN_NO_SPLIT")) return MCMCN_OK;
     const mcmcn_model* e = m->split;
-    const KernelSet* ks = nullptr;
-    int rc = validate(e, s, &ks);
+    const int rc = validate(e, s, &sp.ks);
     if (rc) return rc;
     if (e->n_params != m->n_params || e->n_obs != m->n_obs || e->objective != m->objective || e->precision != m->precision) {
         set_error("split model does not describe the same objective / observations");
         return MCMCN_ERR_INVALID;
     }
     if (!m->split_scratch) { set_error("split_scratch missing"); return MCMCN_ERR_INVALID; }
+    sp.e = e;
+    sp.cand = m->split_scratch;
+    sp.part = sp.cand + (size_t)m->n_params * s->stride;
+    sp.park = sp.part + (size_t)e->n_groups * s->stride;
+    return MCMCN_OK;
+}
+
+// Complete pooling with the observations split into small groups (sp): per sweep propose -> eval over the
+// small groups -> decide.  `mks` is the kernel set of the model m itself (pointwise log-likelihood of the
+// retained rows).
+static int run_complete_split(const KernelSet* mks, const mcmcn_model* m, const Split& sp, const mcmcn_state* s,
+                              const mcmcn_run_args* r, cudaStream_t stream) {
+    const mcmcn_model* e = sp.e;
+    const KernelSet* ks = sp.ks;
     const int P = m->n_params, S = s->stride;
     SweepArgs ea;
     fill_args(ea, ks, e, s);
-    double* cand = m->split_scratch;
-    double* part = cand + (size_t)P * S;
-    double* park = part + (size_t)e->n_groups * S;
-    ea.pooled_theta = cand;
-    ea.out_ll = part;
+    ea.pooled_theta = sp.cand;
+    ea.out_ll = sp.part;
     const Geometry g = geometry(ks, e, s->n_chains);
     ea.tile_bytes = (int)g.tile_bytes;
     const sweep_fn efn = g.wide ? ks->eval_wide : ks->eval_one;
-    rc = set_smem_attr((const void*)efn, g.tile_bytes);
+    int rc = set_smem_attr((const void*)efn, g.tile_bytes);
     if (rc) return rc;
     // linear regression with FP32 observation math: the evaluation runs on the tensor core (eval_tc_kernel),
     // one partial log-likelihood per group RANGE instead of one per small group
@@ -322,8 +339,8 @@ static int run_complete_split(const KernelSet* mks, const mcmcn_model* m, const 
         ta.tc_group_off = reinterpret_cast<const long long*>(e->tc_group_off);
         ta.group_nobs = e->group_nobs;
         ta.bbar = e->obj_const;
-        ta.cand = cand;
-        ta.part = part;
+        ta.cand = sp.cand;
+        ta.part = sp.part;
         ta.P = P; ta.G = e->n_groups; ta.n_chains = s->n_chains; ta.S = S;
         ta.tc_stage_bytes = sb;
         tfn = tc_eval_kernel(e->n_coef > 8 ? 2 : 1);
@@ -336,7 +353,7 @@ static int run_complete_split(const KernelSet* mks, const mcmcn_model* m, const 
     c.P = P; c.n_chains = s->n_chains; c.S = S; c.n_parts = etc ? (int)tg.grid.x : e->n_groups;
     c.chain_id0 = s->chain_id0; c.seed = r->seed;
     c.theta = s->theta; c.scale = s->scale; c.counts = s->counts; c.ll = s->ll; c.lprior = s->lprior;
-    c.cand = cand; c.part = part; c.park = park;
+    c.cand = sp.cand; c.part = sp.part; c.park = sp.park;
     const size_t per_iter = (size_t)P * S;                              // the one group of complete pooling
     int64_t row = r->store_row0;
     KernelTimer tm = {r->timing, stream, false};                        // launch counts only
@@ -402,7 +419,10 @@ int mcmcn_run(const mcmcn_model* m, const mcmcn_state* s, const mcmcn_run_args* 
     if (partial && m->n_groups < 2) { set_error("partial pooling needs at least 2 groups"); return MCMCN_ERR_INVALID; }
     if (partial && r->tape_z && (!r->tape_zmu || !r->tape_qsig)) { set_error("replay of partial pooling needs tape_zmu/tape_qsig"); return MCMCN_ERR_INVALID; }
     cudaStream_t stream = (cudaStream_t)stream_;
-    if (m->pooling == MCMCN_POOL_COMPLETE && m->split && !getenv("MCMCN_NO_SPLIT")) return run_complete_split(ks, m, s, r, stream);
+    Split sp;
+    rc = resolve_split(m, s, sp);
+    if (rc) return rc;
+    if (sp.e) return run_complete_split(ks, m, sp, s, r, stream);
 
     SweepArgs a;
     fill_args(a, ks, m, s);
@@ -506,23 +526,36 @@ int mcmcn_group_loglik(const mcmcn_model* m, const mcmcn_state* s, const double*
     int rc = validate(m, s, &ks);
     if (rc) return rc;
     if (!out_ll) { set_error("null output"); return MCMCN_ERR_INVALID; }
+    Split sp;
+    rc = resolve_split(m, s, sp);
+    if (rc) return rc;
+    const mcmcn_model* em = m;                                          // the model whose groups are evaluated
+    double* eout = out_ll;
+    if (sp.e) {                 // complete pooling at scale: the small groups into split_scratch, added up below
+        em = sp.e;
+        ks = sp.ks;
+        eout = sp.part;
+        if (!pooled_theta) pooled_theta = s->theta;                     // G = 1: [P][1][S] is [P][S]
+    }
+    cudaStream_t stream = (cudaStream_t)stream_;
     SweepArgs a;
-    fill_args(a, ks, m, s);
+    fill_args(a, ks, em, s);
     a.pooled_theta = pooled_theta;
-    a.out_ll = out_ll;
-    const Geometry g = geometry(ks, m, s->n_chains);
+    a.out_ll = eout;
+    const Geometry g = geometry(ks, em, s->n_chains);
     a.tile_bytes = (int)g.tile_bytes;
     const sweep_fn fn = g.wide ? ks->eval_wide : ks->eval_one;
     rc = set_smem_attr((const void*)fn, g.tile_bytes);
     if (rc) return rc;
-    CK(launch_sweep(fn, g.grid, g.block, g.tile_bytes, (cudaStream_t)stream_, a));
+    CK(launch_sweep(fn, g.grid, g.block, g.tile_bytes, stream, a));
+    if (sp.e) group_sum_kernel<false><<<(s->stride + 127) / 128, 128, 0, stream>>>(sp.e->n_groups, s->stride, sp.part, out_ll);
     CK(cudaGetLastError());
     return MCMCN_OK;
 }
 
 int mcmcn_pooled_nll(int n_groups, int stride, const double* ll, double* out, void* stream_) {
     if (n_groups < 1 || stride < 1 || !ll || !out) { set_error("bad pooled_nll args"); return MCMCN_ERR_INVALID; }
-    pooled_nll_kernel<<<(stride + 127) / 128, 128, 0, (cudaStream_t)stream_>>>(n_groups, stride, ll, out);
+    group_sum_kernel<true><<<(stride + 127) / 128, 128, 0, (cudaStream_t)stream_>>>(n_groups, stride, ll, out);
     CK(cudaGetLastError());
     return MCMCN_OK;
 }

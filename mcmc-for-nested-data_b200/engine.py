@@ -13,6 +13,7 @@ import ctypes
 import os
 import threading
 import time
+import types
 
 import numpy
 import scipy.special
@@ -46,6 +47,11 @@ def _retainedRange(lo, hi, burn, thin):
 def retainedIterations(nIter, burn, thin):
     """Iterations whose state Sampler._loop writes out (:887)."""
     return list(_retainedRange(0, nIter, burn, thin))
+
+
+def retainedCount(lo, hi, burn, thin):
+    """Number of iterations i in [lo, hi) that Sampler._loop retains (i >= burn and i % thin == 0, :887)."""
+    return len(_retainedRange(lo, hi, burn, thin))
 
 
 def hostNormLogpdf(x, loc, scale):
@@ -122,11 +128,6 @@ WRITER_THREADS = _hostThreads("MCMCN_STORE_THREADS")
 # as many as writers: the file's pages are populated while the chains burn in and the writers have nothing to do (C3:
 # 37.8 GB in 2.9 s takes eight threads; with four the writers met unpopulated pages and the sampling phase waited)
 PREFAULT_THREADS = int(os.environ.get("MCMCN_PREFAULT_THREADS", WRITER_THREADS))
-
-
-def retainedCount(lo, hi, burn, thin):
-    """Number of iterations i in [lo, hi) that Sampler._loop retains (i >= burn and i % thin == 0, :887)."""
-    return len(_retainedRange(lo, hi, burn, thin))
 
 
 class SampleStore(object):
@@ -382,13 +383,12 @@ class Engine(object):
         # MCMCN_TASK_OBS: observations per task of the FP32-pipe step kernel (a CTA's run of consecutive groups,
         # staged by one TMA copy); results do not depend on it -- a tuning knob for experiments
         taskObsTarget = int(os.environ.get("MCMCN_TASK_OBS", taskObsTarget))
-        m, keep = self._buildModel(stepped, pooling, taskObsTarget, tensorCore=True)
-        (self._data, self._group_off, self._group_nobs, self._task_group0, self._obj_const, self._tc_data,
-         self._tc_group_off, self._group_off_h, self._task_group0_h) = keep
+        self._main = self._buildModel(stepped, pooling, taskObsTarget)
+        self.model = m = self._main.model
+        self._data = self._main.data
         if not self.partial:
             for p, d in enumerate(priorDistribution):
                 m.prior[p] = priorFromScipy(d)
-        self.model = m
         if objective.kind != nat.OBJ_USER and not self.lib.mcmcn_supported(
                 m.objective, m.n_params, m.n_coef, m.precision):
             raise RuntimeError("objective kind %d with %d parameters (%d coefficients) at %s is not compiled "
@@ -423,44 +423,40 @@ class Engine(object):
             if objective.kind == nat.OBJ_LINEAR_REGRESSION and objective.precision == "fp32":
                 size = 112 if objective.nCoef <= 8 else 96
             parts = [size] * (N // size) + ([N % size] if N % size else [])
-            sm, skeep = self._buildModel(parts, pooling, taskObsTarget, tensorCore=True, commonReference=True)
-            scratch = torch.zeros(((P + len(parts) + 3) * S,), dtype=f64, device=dev)
-            self._split = (sm, skeep, scratch)
-            self.model.split = ctypes.addressof(sm)
-            self.model.split_scratch = _ptr(scratch)
+            self._split = self._buildModel(parts, pooling, taskObsTarget, commonReference=True)
+            self._split.scratch = torch.zeros(((P + len(parts) + 3) * S,), dtype=f64, device=dev)
+            self.model.split = ctypes.addressof(self._split.model)
+            self.model.split_scratch = _ptr(self._split.scratch)
 
-    def _buildModel(self, stepped, pooling, taskObsTarget, tensorCore, commonReference=False):
-        """Pack the objective's observations as the groups `stepped` and describe them as a
-        mcmcn_model (include/mcmcn.h).  Returns the model and the tensors / arrays it points into."""
+    def _buildModel(self, stepped, pooling, taskObsTarget, commonReference=False):
+        """Pack the objective's observations as the groups `stepped` (Objective.pack) and describe them as a
+        mcmcn_model (include/mcmcn.h).  Returns a namespace holding the nat.Model (``model``) and every tensor
+        and host array it points into, so that they live as long as it does; ``data`` and ``tcData`` are the
+        FP32-pipe and tcgen05 observation blocks."""
         objective, dev = self.objective, self.device
+        pk = objective.pack(stepped, commonReference)
         nG = len(stepped)
-        data, group_off, group_nobs, obj_const = objective.pack(stepped, commonReference) \
-            if commonReference else objective.pack(stepped)
-        elem = data.dtype.itemsize
-        cap = self.lib.mcmcn_tile_capacity_bytes() // elem
+        cap = self.lib.mcmcn_tile_capacity_bytes() // pk.data.dtype.itemsize
         task_group0 = [0]
         acc_elems, acc_obs = 0, 0
         for g in range(nG):
-            e = int(group_off[g + 1] - group_off[g])
-            if g > task_group0[-1] and (acc_elems + e > cap or acc_obs + int(group_nobs[g]) > taskObsTarget):
+            e = int(pk.groupOff[g + 1] - pk.groupOff[g])
+            if g > task_group0[-1] and (acc_elems + e > cap or acc_obs + int(pk.groupNobs[g]) > taskObsTarget):
                 task_group0.append(g)
                 acc_elems, acc_obs = 0, 0
             acc_elems += e
-            acc_obs += int(group_nobs[g])
+            acc_obs += int(pk.groupNobs[g])
         task_group0.append(nG)
-        group_off_h = numpy.ascontiguousarray(group_off, dtype=numpy.int64)
-        task_group0_h = numpy.ascontiguousarray(task_group0, dtype=numpy.int32)
-        d_data = torch.from_numpy(data).to(dev)
-        d_group_off = torch.from_numpy(group_off_h).to(dev)
-        d_group_nobs = torch.from_numpy(group_nobs).to(dev)
-        d_task_group0 = torch.from_numpy(task_group0_h).to(dev)
-        d_obj_const = torch.from_numpy(obj_const).to(dev) if obj_const is not None else None
-        tcData = getattr(objective, "tcData", None) if tensorCore else None
-        tcOff = getattr(objective, "tcGroupOff", None) if tensorCore else None
-        d_tc_data = torch.from_numpy(tcData).to(dev) if tcData is not None else None
-        d_tc_group_off = torch.from_numpy(tcOff).to(dev) if tcData is not None else None
 
-        m = nat.Model()
+        def up(a):
+            return torch.from_numpy(a).to(dev) if a is not None else None
+        b = types.SimpleNamespace(groupOffHost=numpy.ascontiguousarray(pk.groupOff, dtype=numpy.int64),
+                                  taskGroup0Host=numpy.ascontiguousarray(task_group0, dtype=numpy.int32))
+        b.data, b.groupOff, b.groupNobs = up(pk.data), up(b.groupOffHost), up(pk.groupNobs)
+        b.taskGroup0, b.objConst = up(b.taskGroup0Host), up(pk.objConst)
+        b.tcData, b.tcGroupOff = up(pk.tcData), up(pk.tcGroupOff)
+
+        m = b.model = nat.Model()
         m.objective = objective.kind
         m.n_params = self.P
         m.n_coef = objective.nCoef
@@ -468,20 +464,19 @@ class Engine(object):
         m.pooling = nat.POOLING_CODE[pooling]
         m.n_groups = nG
         m.n_tasks = len(task_group0) - 1
-        m.n_obj_const = 0 if obj_const is None else len(obj_const)
+        m.n_obj_const = 0 if pk.objConst is None else len(pk.objConst)
         m.n_obs = self.nObservations
-        m.data = _ptr(d_data)
-        m.group_off = _ptr(d_group_off)
-        m.group_nobs = _ptr(d_group_nobs)
-        m.task_group0 = _ptr(d_task_group0)
-        m.task_group0_host = task_group0_h.ctypes.data_as(ctypes.c_void_p)
-        m.group_off_host = group_off_h.ctypes.data_as(ctypes.c_void_p)
-        m.obj_const = _ptr(d_obj_const)
+        m.data = _ptr(b.data)
+        m.group_off = _ptr(b.groupOff)
+        m.group_nobs = _ptr(b.groupNobs)
+        m.task_group0 = _ptr(b.taskGroup0)
+        m.task_group0_host = b.taskGroup0Host.ctypes.data_as(ctypes.c_void_p)
+        m.group_off_host = b.groupOffHost.ctypes.data_as(ctypes.c_void_p)
+        m.obj_const = _ptr(b.objConst)
         m.user_objective = objective.userHandle
-        m.tc_data, m.tc_group_off = _ptr(d_tc_data), _ptr(d_tc_group_off)
-        m.tc_max_block_floats = int(numpy.diff(tcOff).max()) if tcData is not None else 0
-        return m, (d_data, d_group_off, d_group_nobs, d_task_group0, d_obj_const, d_tc_data, d_tc_group_off,
-                   group_off_h, task_group0_h)
+        m.tc_data, m.tc_group_off = _ptr(b.tcData), _ptr(b.tcGroupOff)
+        m.tc_max_block_floats = int(numpy.diff(pk.tcGroupOff).max()) if pk.tcData is not None else 0
+        return b
 
     # ------------------------------------------------------------------ helpers
     @property
@@ -492,13 +487,13 @@ class Engine(object):
     @property
     def stepInput(self):
         """The device tensor of observation data the step kernel reads."""
-        return self._tc_data if self.usesTensorCore else self._data
+        return self._main.tcData if self.usesTensorCore else self._data
 
     @property
     def stream(self):
         return ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
-    def _up(self, dst, src, lastAxisChains=True):
+    def _up(self, dst, src):
         """Copy a host array whose last axis is the chain into a [.., S] device tensor."""
         t = torch.from_numpy(numpy.ascontiguousarray(src)).to(self.device)
         dst[..., :self.nChains].copy_(t.to(dst.dtype))
@@ -544,24 +539,13 @@ class Engine(object):
     # ------------------------------------------------------------------ evaluation
     def groupLogLikelihood(self, pooledTheta=None):
         """[G][S] device tensor of group log-likelihoods of the current state, or of
-        ``pooledTheta`` ([P][nChains] host array: every group uses the same values)."""
+        ``pooledTheta`` ([P][nChains] host array: every group uses the same values).  Lanes from
+        nChains on are unspecified."""
         out = torch.empty((self.G, self.S), dtype=torch.float64, device=self.device)
         pt = None
         if pooledTheta is not None:
             pt = torch.zeros((self.P, self.S), dtype=torch.float64, device=self.device)
             self._up(pt, pooledTheta)
-        if self._split is not None and not os.environ.get("MCMCN_NO_SPLIT"):
-            # complete pooling at scale: evaluate over the groups of 128 in parallel and add them up in
-            # group order (the single stepped group's current values are themselves a pooled vector);
-            # the start-state search and the MLE start call this hundreds of times
-            sm = self._split[0]
-            if pt is None:
-                pt = self.theta[:, 0, :].contiguous()
-            parts = torch.zeros((sm.n_groups, self.S), dtype=torch.float64, device=self.device)
-            nat.call("mcmcn_group_loglik", ctypes.byref(sm), ctypes.byref(self.state), _ptr(pt), _ptr(parts), self.stream)
-            nll = torch.zeros((self.S,), dtype=torch.float64, device=self.device)
-            nat.call("mcmcn_pooled_nll", int(sm.n_groups), self.S, _ptr(parts), _ptr(nll), self.stream)
-            return nll.neg_().reshape(1, self.S)
         nat.call("mcmcn_group_loglik", ctypes.byref(self.model), ctypes.byref(self.state),
                  _ptr(pt), _ptr(out), self.stream)
         return out

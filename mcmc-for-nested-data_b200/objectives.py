@@ -13,6 +13,8 @@ Registry (device code in csrc/mcmcn_device.cuh):
   bernoulli_logit         SURVEY.md config C5
 """
 
+import collections
+
 import numpy
 
 import mcmcn_native as nat
@@ -20,6 +22,13 @@ import mcmcn_native as nat
 
 def _round4(n):
     return (int(n) + 3) & ~3
+
+
+# What Objective.pack makes of the observations (include/mcmcn.h, mcmcn_model): ``data`` one block per stepped
+# group for the FP32-pipe kernels, ``groupOff`` [G+1] block offsets, ``groupNobs`` [G] observations per group,
+# ``objConst`` the objective constants or None, ``tcData`` / ``tcGroupOff`` the tcgen05 operand blocks and their
+# offsets (linear regression in FP32 with K <= 16; None otherwise).
+Packed = collections.namedtuple("Packed", "data groupOff groupNobs objConst tcData tcGroupOff")
 
 
 class Objective(object):
@@ -132,7 +141,7 @@ class Objective(object):
         the least-squares fit over all observations, instead of its own fit -- what complete pooling
         split over observations wants: the chain's one candidate vector then has one centred form for
         every small group.
-        Returns (data, group_off[G+1], group_nobs[G], obj_const or None)."""
+        Returns a Packed record."""
         nResp = [int(r) for r in nResponsesPerGroup]
         if sum(nResp) != self.nObservations:
             raise ValueError("nResponsesPerGroup sums to %d but the objective holds %d observations"
@@ -155,7 +164,7 @@ class Objective(object):
                 rec = blk[H:].reshape(r, F)
                 rec[:, :self.records.shape[1]] = self.records[start:start + r]
                 start += r
-            return data, group_off, numpy.array(nResp, dtype=numpy.int32), None
+            return Packed(data, group_off, numpy.array(nResp, dtype=numpy.int32), None, None, None)
         if self.kind == nat.OBJ_LINEAR_REGRESSION:
             K, KP = self.nCoef, _round4(self.nCoef)
             unit = 4 * KP + 4
@@ -205,15 +214,14 @@ class Objective(object):
                 ms[:r, :P] = self.mu[:, self.groupOfObservation[rows]].T
                 blk[:, :] = ms.reshape(q, 4 * PP)
             start += r
-        obj_const = None
-        self.tcData = self.tcGroupOff = None
+        obj_const = tcData = tcGroupOff = None
         if self.kind == nat.OBJ_LINEAR_REGRESSION:
             obj_const = numpy.ascontiguousarray(bbar.reshape(-1))
             if self.precision == "fp32" and self.nCoef <= 16:
-                self.tcData, self.tcGroupOff = self._packTensorCore(nResp, bbar)
+                tcData, tcGroupOff = self._packTensorCore(nResp, bbar)
         if self.kind == nat.OBJ_GAUSSIAN_DISTRIBUTION:
             obj_const = numpy.concatenate([self.sd, numpy.log(self.sd)]).astype(numpy.float64)
-        return data, group_off, numpy.array(nResp, dtype=numpy.int32), obj_const
+        return Packed(data, group_off, numpy.array(nResp, dtype=numpy.int32), obj_const, tcData, tcGroupOff)
 
     def _packTensorCore(self, nResp, bbar):
         """Operand blocks of the tcgen05 step kernel (include/mcmcn.h, mcmcn_model.tc_data): per group the

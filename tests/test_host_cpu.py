@@ -105,7 +105,8 @@ def test_regression_packing_is_the_same_residual():
     N, K = sum(nResp), 3
     X, y = rs.normal(size=(N, K)), 100 + rs.normal(size=N)
     for prec in ("fp32", "fp64"):
-        data, off, nobs, bbar = Objective.linear_regression(X, y, prec).pack(nResp)
+        pk = Objective.linear_regression(X, y, prec).pack(nResp)
+        data, off, nobs, bbar = pk.data, pk.groupOff, pk.groupNobs, pk.objConst
         KP, unit = 4, 4 * 4 + 4
         bbar = bbar.reshape(len(nResp), K)
         start = 0
@@ -134,7 +135,8 @@ def test_split_packing_of_complete_pooling_is_the_same_sum_of_squares():
     b = rs.normal(size=K)
     want = float(numpy.sum((X @ b - y) ** 2))
     for stepped in ([N], [128, 128, 44]):
-        data, off, nobs, bbar = obj.pack(stepped)
+        pk = obj.pack(stepped)
+        data, off, nobs, bbar = pk.data, pk.groupOff, pk.groupNobs, pk.objConst
         bbar = bbar.reshape(len(stepped), K)
         unit, total = 4 * 4 + 4, 0.0
         for g in range(len(stepped)):
@@ -155,8 +157,8 @@ def test_tensor_core_operand_blocks_are_an_exact_3xtf32_split():
     N, K = sum(nResp), 5
     X, y = rs.normal(size=(N, K)), 300 + rs.normal(size=N)
     obj = Objective.linear_regression(X, y, "fp32")
-    data, off, nobs, bbar = obj.pack(nResp)
-    tc, tcOff = obj.tcData, obj.tcGroupOff
+    pk = obj.pack(nResp)
+    bbar, tc, tcOff = pk.objConst, pk.tcData, pk.tcGroupOff
     assert tc.dtype == numpy.float32 and len(tcOff) == len(nResp) + 1
     assert numpy.all((tc.view(numpy.uint32) & 0x1FFF) == 0)              # exact in TF32
     bbar = bbar.reshape(len(nResp), K)
@@ -180,6 +182,27 @@ def test_tensor_core_operand_blocks_are_an_exact_3xtf32_split():
         for (i, k) in ((0, 0), (r - 1, K - 1), (9 % n, 4)):
             assert blk[(i // 8) * 64 + (k // 4) * 32 + (i % 8) * 4 + (k % 4)] == xhi[i, k]
         start += r
+
+
+def test_packing_returns_one_record_and_leaves_the_objective_as_it_was():
+    """Objective.pack hands everything it packs back in its record (also the tensor-core operand
+    blocks, which exist for linear regression in FP32 with K <= 16 only) and sets nothing on the
+    objective, so that packing the same objective twice (complete pooling at scale) cannot mix the
+    two results."""
+    from objectives import Objective
+    rs = numpy.random.RandomState(2)
+    N = 300
+    x, y = rs.normal(size=N), (rs.uniform(size=N) < 0.5).astype(float)
+    cases = [(Objective.linear_regression(rs.normal(size=(N, K)), y, prec), K <= 16 and prec == "fp32")
+             for K in (2, 16, 17) for prec in ("fp32", "fp64")]
+    cases.append((Objective.bernoulli_logit(x, y), False))
+    for obj, hasTc in cases:
+        before = dict(vars(obj))
+        for pk in (obj.pack([N]), obj.pack([128, 128, 44], commonReference=True)):
+            assert vars(obj).keys() == before.keys() and all(vars(obj)[k] is v for k, v in before.items())
+            assert (pk.tcData is not None) == hasTc and (pk.tcGroupOff is not None) == hasTc
+            if hasTc:
+                assert pk.tcGroupOff[-1] == pk.tcData.size and len(pk.tcGroupOff) == len(pk.groupNobs) + 1
 
 
 def test_prior_mapping():
